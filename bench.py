@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- grid-cell-timesteps/s on the fused PV convert+aggregate path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload = the BASELINE.json north star: synthetic ERA5 1440 x 720 x 8760
 (global 0.25 deg, one year hourly), cutout.pv(panel="CSi",
@@ -31,6 +31,14 @@ cutout), and every step ends with the NCCL all-gather that re-assembles the
 `extra`   : BASELINE configs[2] (wind) and configs[3] (heat demand) on the same
             grid and shards, same protocol (strong scaling at N > 1); at N = 1
             also configs[1], the non-default PV variants, config 4, the indicator matrix.
+
+`--steps K` is the number of timed passes of the headline, of `e2e` and of the wind /
+heat entries of `extra`; `--warmup W` untimed passes precede those of the headline and
+of wind / heat.  `--dump-outputs DIR` then writes the (time, bus) results of the last
+timed pass of the headline (`pv`) and of wind and heat demand as float32
+`DIR/<name>.npy`, with the time steps they hold in `DIR/<name>_time_index.npy`, 64 MB
+in all (see `dump_outputs`).  The inputs are seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 
 from __future__ import annotations
@@ -54,6 +62,8 @@ PANEL, ORIENT, TURBINE = "CSi", "latitude_optimal", "Vestas_V112_3MW"
 BYTES_PER_CELL_TS = 20.0  # 5 float32 fields (SURVEY.md section 8d)
 E2E_MAX_STEPS = 1095  # host-streamed slab per rank (22.7 GB of pinned host memory)
 VRAM_FRACTION = 0.80  # share of the device memory the resident inputs may take
+DUMP_BYTES = 64_000_000  # --dump-outputs: every file together, headers included
+DUMP_SEED = 0
 WORKLOAD = (f"synthetic ERA5 {NX}x{NY}x{NT}, cutout.pv(panel=CSi, orientation=latitude_optimal) "
             f"-> {NBUS} shapes (BASELINE.json north star)")
 METRIC = "grid-cell-timesteps/s on PV convert+aggregate"
@@ -441,6 +451,26 @@ def check_gather(comm, res, lo, hi):
     return True
 
 
+def dump_outputs(outdir, results):
+    """Write each (time, bus) result as float32 `outdir/<name>.npy` and the time steps it holds
+    as float64 `outdir/<name>_time_index.npy`, in at most DUMP_BYTES together.  Results are
+    kept whole smallest first while they fit an equal share of what is left; a larger one keeps
+    a sorted sample of its time steps drawn with DUMP_SEED, so the same shapes give the same
+    sample on every run."""
+    os.makedirs(outdir, exist_ok=True)
+    left = DUMP_BYTES - 2 * 4096 * len(results)  # 4 KiB per .npy header is generous (NumPy writes 128 B)
+    row_bytes = {k: v.shape[1] * 4 + 8 for k, v in results.items()}  # float32 row + its float64 index
+    order = sorted(results, key=lambda k: results[k].shape[0] * row_bytes[k])
+    for i, name in enumerate(order):
+        v = results[name]
+        n = v.shape[0]
+        keep = min(n, left // (len(order) - i) // row_bytes[name])
+        left -= keep * row_bytes[name]
+        rows = np.arange(n) if keep == n else np.sort(np.random.default_rng(DUMP_SEED).choice(n, keep, replace=False))
+        np.save(os.path.join(outdir, f"{name}.npy"), np.ascontiguousarray(v[rows], dtype=np.float32))
+        np.save(os.path.join(outdir, f"{name}_time_index.npy"), rows.astype(np.float64))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -481,7 +511,7 @@ def run_ours(args):
 
     def run_parts(parts):
         bounds = [(lo + (hi - lo) * p // parts, lo + (hi - lo) * (p + 1) // parts) for p in range(parts)]
-        acc = {"ms_step": 0.0, "kern_ms": 0.0, "kern_ranks": [0.0] * world, "gather_ms": None}
+        acc = {"ms_step": 0.0, "kern_ms": 0.0, "kern_ranks": [0.0] * world, "gather_ms": None, "last": []}
         for p, (a, b) in enumerate(bounds):
             f = syn.make_pv_fields_device(time_axis[a:b], x, y, dev, seed=0, t_offset=a)
             spec = _PvSpec(ab.Dataset(f, coords=dict(time=time_axis[a:b], **co)),
@@ -497,6 +527,8 @@ def run_ours(args):
             acc["kern_ms"] += res["kernel_ms"]
             acc["kern_ranks"] = [u + v for u, v in zip(acc["kern_ranks"], res["kernel_ms_per_rank"])]
             acc["gather_ms"] = res["gather_ms"]
+            if args.dump_outputs:
+                acc["last"].append(res["full"].cpu())
             del f, spec, res
             torch.cuda.empty_cache()
         return acc
@@ -512,6 +544,7 @@ def run_ours(args):
             parts += 1
             torch.cuda.empty_cache()
     ms_step, kern_ms, kern_ranks, gather_ms = acc["ms_step"], acc["kern_ms"], acc["kern_ranks"], acc["gather_ms"]
+    outputs = {"pv": torch.cat(acc["last"]).numpy()} if args.dump_outputs else None
     launches = _lib.launch_count() - n0
     value = S * NT / (ms_step * 1e-3)
     cell_ts_local = S * (hi - lo)
@@ -548,15 +581,14 @@ def run_ours(args):
     def step_e2e():
         return cut_host.pv(PANEL, ORIENT, matrix=shapes, aggregate_time=None)
 
-    e2e_steps = max(2, min(args.steps, 3))
     res = step_e2e()
     comm.sync()
     t0 = time.perf_counter()
-    for _ in range(e2e_steps):
+    for _ in range(args.steps):
         res = step_e2e()
     torch.cuda.synchronize()
     e2e_s = comm.max(time.perf_counter() - t0)
-    e2e_value = S * ne * world * e2e_steps / e2e_s
+    e2e_value = S * ne * world * args.steps / e2e_s
     api_res = np.asarray(res.values).T
     agree = float(np.max(np.abs(dev_slab - api_res) / (np.abs(api_res) + 1e-3)))
     del host, cut_host, res
@@ -582,7 +614,7 @@ def run_ours(args):
                         if world > 1 else {})},
         "e2e": {"value": e2e_value, "unit": "grid-cell-timesteps/s",
                 "h2d_bytes_per_step": int(S * ne * BYTES_PER_CELL_TS),
-                "d2h_bytes_per_step": int(ne * NBUS * 4), "steps": e2e_steps,
+                "d2h_bytes_per_step": int(ne * NBUS * 4), "steps": args.steps,
                 "sample": f"each rank streams the first {ne} steps of its shard from pinned host memory "
                           f"({world * ne} of {NT} steps per pass)",
                 "api": "atlite_b200.Cutout(data=<pinned host arrays>).pv('CSi','latitude_optimal',matrix=...,aggregate_time=None)",
@@ -597,11 +629,13 @@ def run_ours(args):
     # ---- BASELINE configs[2] / configs[3] on the same grid and shards
     extra = {}
     if not args.no_extra:
-        extra.update(wind_heat_sharded(comm, shard, plan, x, y, time_axis, args, peak))
+        extra.update(wind_heat_sharded(comm, shard, plan, x, y, time_axis, args, peak, outputs))
         if world == 1:
             extra.update(extra_single_gpu(torch, dev, peak))
     if extra:
         line["extra"] = extra
+    if rank == 0 and outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     if rank == 0 and world == 1:
         line["cpu_baseline"] = cpu_baseline()
     if rank == 0:
@@ -610,11 +644,12 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
-def wind_heat_sharded(comm, shard, plan, x, y, time_axis, args, peak):
+def wind_heat_sharded(comm, shard, plan, x, y, time_axis, args, peak, outputs=None):
     """BASELINE configs[2] (wind, Vestas V112 3 MW) and configs[3] (heat demand) on the
     1440 x 720 x 8760 cutout -> 3000 shapes: this rank's time shard resident in HBM, same
     timed region as the headline (strong scaling at N > 1).  Heat-demand shards are cut on
-    day boundaries (dist.shard_bounds(align=24)), so they may differ by one day."""
+    day boundaries (dist.shard_bounds(align=24)), so they may differ by one day.  The full
+    (time, bus) results of the last timed passes go into `outputs` when it is a dict."""
     import atlite_b200 as ab
     from atlite_b200 import synthetic as syn
     from atlite_b200.convert import _HeatSpec, _WindSpec
@@ -624,7 +659,6 @@ def wind_heat_sharded(comm, shard, plan, x, y, time_axis, args, peak):
     S = float(NX) * NY
     world, rank = comm.world, comm.rank
     out = {}
-    steps = max(3, min(args.steps, 5))
 
     def entry(r, n_local, bytes_per):
         return {"cell_ts_per_s": S * NT / (r["ms_per_step"] * 1e-3), "ms_per_step": r["ms_per_step"],
@@ -637,9 +671,12 @@ def wind_heat_sharded(comm, shard, plan, x, y, time_axis, args, peak):
     co = dict(time=time_axis[lo:hi], x=x, y=y, lon=x, lat=y)
     f = syn.make_wind_fields_device(hi - lo, NY, NX, comm.dev, seed=1, t_offset=lo)
     ws = _WindSpec(ab.Dataset(f, coords=co), ab.get_windturbineconfig(TURBINE))
-    r = measure_sharded(comm, shard, lambda: ws.op.reduce(plan, ws.wnd, ws.aux), (hi - lo) * S, counts, steps, 2)
+    r = measure_sharded(comm, shard, lambda: ws.op.reduce(plan, ws.wnd, ws.aux), (hi - lo) * S, counts,
+                        args.steps, args.warmup)
     if shard is not None:
         check_gather(comm, r, sum(counts[:rank]), sum(counts[:rank + 1]))
+    if outputs is not None:
+        outputs["wind"] = r["full"].cpu().numpy()
     out["wind_c2_1440x720x8760_3000"] = entry(r, hi - lo, 8)
     if world == 1:
         # the same kernel on a quarter-year slab (what each rank of a 4-GPU run processes): the 72.6 GB
@@ -662,9 +699,12 @@ def wind_heat_sharded(comm, shard, plan, x, y, time_axis, args, peak):
     co = dict(time=time_axis[lo:hi], x=x, y=y, lon=x, lat=y)
     tf = syn.make_pv_fields_device(time_axis[lo:hi], x, y, comm.dev, seed=2, names=("temperature",), t_offset=lo)
     hs = _HeatSpec(ab.Dataset(tf, coords=co), 15.0, 1.0, 0.0, 0.0)
-    r = measure_sharded(comm, shard, lambda: hs.op.reduce(plan, hs.temp, hs.day_start), (hi - lo) * S, dcounts, steps, 2)
+    r = measure_sharded(comm, shard, lambda: hs.op.reduce(plan, hs.temp, hs.day_start), (hi - lo) * S, dcounts,
+                        args.steps, args.warmup)
     if shard is not None:
         check_gather(comm, r, sum(dcounts[:rank]), sum(dcounts[:rank + 1]))
+    if outputs is not None:
+        outputs["heat_demand"] = r["full"].cpu().numpy()
     out["heat_c3_1440x720x8760_3000"] = entry(r, hi - lo, 4)
     out["heat_c3_1440x720x8760_3000"]["days_per_rank"] = dcounts
     del hs, r, tf
@@ -780,7 +820,13 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-extra", action="store_true", help="skip the configs[2,3] / variant roofline points")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the (time, bus) results of the last timed pass to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -6,6 +6,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -32,3 +35,33 @@ def test_reference_arm_other_ranks_exit_quietly():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2",
                         "--steps", "1", "--warmup", "0"], capture_output=True, text=True, timeout=300, env=env)
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--warmup", "-1"],
+                                  ["--impl", "reference", "--dump-outputs", "out"]])
+def test_bad_arguments_are_refused(argv, tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, capture_output=True, text=True,
+                       timeout=120, cwd=tmp_path)
+    assert r.returncode == 2 and "error" in r.stderr
+    assert not os.listdir(tmp_path)
+
+
+def test_dump_outputs_fits_the_budget_with_a_fixed_sample(tmp_path, monkeypatch):
+    import bench
+
+    monkeypatch.setattr(bench, "DUMP_BYTES", 1 << 20)
+    rng = np.random.default_rng(3)
+    results = {"pv": rng.random((1000, 300)), "wind": rng.random((1000, 300), dtype=np.float32),
+               "heat_demand": rng.random((40, 300), dtype=np.float32)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), results)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == sorted(f"{k}{s}.npy" for k in results for s in ("", "_time_index"))
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= bench.DUMP_BYTES
+    for k, v in results.items():
+        got, rows = np.load(tmp_path / "a" / f"{k}.npy"), np.load(tmp_path / "a" / f"{k}_time_index.npy")
+        assert got.dtype == np.float32 and rows.dtype == np.float64
+        assert np.array_equal(got, v[rows.astype(np.int64)].astype(np.float32))
+        assert np.array_equal(got, np.load(tmp_path / "b" / f"{k}.npy"))  # the same sample on every run
+    assert len(np.load(tmp_path / "a" / "heat_demand_time_index.npy")) == 40  # small results stay whole
+    assert 0 < len(np.load(tmp_path / "a" / "pv_time_index.npy")) < 1000
