@@ -102,27 +102,50 @@ def _to_host(a):
 # --------------------------------------------------------------------------
 
 
+def _solar_source(ds):
+    """SolarPosition: getter vs computation (pv/solar_position.py:54-67) -> (SOLAR_* value,
+    names of the stored solar position fields)."""
+    if _has(ds, "solar_azimuth") and _has(ds, "solar_altitude"):
+        dt = np.dtype(str(_raw(ds, "solar_altitude").dtype).replace("torch.", ""))
+        return (_lib.SOLAR_STORED_F64 if dt == np.float64 else _lib.SOLAR_STORED_F32), \
+            ["solar_altitude", "solar_azimuth"]
+    warnings.warn(_SOLAR_WARNING, DeprecationWarning)
+    return _lib.SOLAR_COMPUTED, []
+
+
 class _Spec:
     """A known conversion bound to a cutout: can reduce to buses, or produce
-    per-cell values / their time sum."""
+    per-cell values / their time sum.  A subclass sets its operator ``op`` and its
+    input ``fields`` (name -> (time, y, x) array or None, through ``_set_fields``)."""
 
     time_labels = None  # output time coordinate
     name = None
     units = None
 
-    def _device_fields(self, fields):
+    def __init__(self, ds):
+        self.ny, self.nx = _grid_shape(ds)
+        self.time_labels = pd.DatetimeIndex(_coord(ds, "time"))
+
+    def _set_fields(self, fields):
+        self.fields = fields
+        self.pitch = engine.pitch_of(fields.values(), self.nx)
+
+    def _device_fields(self):
         """Host arrays -> device tensors (per-cell output paths only)."""
         torch = engine._torch()
         dev = f"cuda:{engine.current_device()}"
         return {
             k: (v if v is None or engine._is_torch(v) else torch.from_numpy(np.ascontiguousarray(v)).to(dev))
-            for k, v in fields.items()
+            for k, v in self.fields.items()
         }
 
-    def cells_timesum(self):
-        """(NaN-skipping per-cell time sum, number of valid steps per cell), each (y, x)."""
-        sc = self.cells(timesum=True)
-        return sc[0], sc[1]
+    def reduce(self, plan):
+        return self.op.reduce(plan, self.fields)
+
+    def cells(self, timesum=False):
+        """Per-cell values (time, y, x), or with ``timesum`` the NaN-skipping per-cell time sum
+        and the number of valid steps per cell, stacked (2, y, x)."""
+        return self.op.cells(self._device_fields(), timesum=timesum)
 
 
 class _PvSpec(_Spec):
@@ -130,18 +153,11 @@ class _PvSpec(_Spec):
 
     def __init__(self, ds, panel, orientation, tracking=None, trigon_model="simple",
                  clearsky_model="simple", output="panel", thermal=(0.0, 0.0, 0.0)):
-        ny, nx = _grid_shape(ds)
+        super().__init__(ds)
+        ny, nx = self.ny, self.nx
         self.ds = ds
-        self.time_labels = pd.DatetimeIndex(_coord(ds, "time"))
         lon, lat = _coord(ds, "lon").astype(np.float64), _coord(ds, "lat").astype(np.float64)
-
-        # SolarPosition: getter vs computation (pv/solar_position.py:54-67)
-        if _has(ds, "solar_azimuth") and _has(ds, "solar_altitude"):
-            dt = np.dtype(str(_raw(ds, "solar_altitude").dtype).replace("torch.", ""))
-            solar_src = _lib.SOLAR_STORED_F64 if dt == np.float64 else _lib.SOLAR_STORED_F32
-        else:
-            warnings.warn(_SOLAR_WARNING, DeprecationWarning)
-            solar_src = _lib.SOLAR_COMPUTED
+        solar_src, solar_names = _solar_source(ds)
 
         # SurfaceOrientation (pv/orientation.py:104-109, 177-183)
         if tracking not in _lib.TRACKING:
@@ -211,23 +227,15 @@ class _PvSpec(_Spec):
         if irr_branch == _lib.IRR_INFLUX and clearsky == 1:
             names.append("humidity")
         names.append("albedo" if albedo_src == _lib.ALBEDO_VAR else "outflux")
-        if solar_src != _lib.SOLAR_COMPUTED:
-            names += ["solar_altitude", "solar_azimuth"]
-        self.fields = {n: _raw(ds, n) for n in names}
-        self.fields.setdefault("temperature", self.fields["influx_toa"])  # unused placeholder
-        self.pitch = engine.pitch_of(self.fields.values(), nx)
+        fields = {n: _raw(ds, n) for n in names + solar_names}
+        fields.setdefault("temperature", fields["influx_toa"])  # unused placeholder
+        self._set_fields(fields)
         self.op = engine.PvOp(
             ny=ny, nx=nx, time=self.time_labels, lon=lon, lat=lat, slope=slope, azimuth=azimuth,
             tracking=tracking, trigon_model=trigon, clearsky_model=clearsky,
             irr_branch=irr_branch, albedo_src=albedo_src, solar_src=solar_src, panel=panel,
             output=output, thermal=thermal, pitch=self.pitch,
         )
-
-    def reduce(self, plan):
-        return self.op.reduce(plan, self.fields)
-
-    def cells(self, timesum=False):
-        return self.op.cells(self._device_fields(self.fields), timesum=timesum)
 
 
 class _IrradiationSpec(_PvSpec):
@@ -256,22 +264,13 @@ class _PointwiseSpec(_Spec):
     """Pointwise function of one (time, y, x) variable."""
 
     def __init__(self, ds, var, shift=0.0, nan_to_zero=False, poly=None, cell_scale=None, name=None):
-        ny, nx = _grid_shape(ds)
+        super().__init__(ds)
         if not _has(ds, var):
             raise KeyError(var)
-        self.field = _raw(ds, var)
-        self.time_labels = pd.DatetimeIndex(_coord(ds, "time"))
+        self._set_fields({var: _raw(ds, var)})
         self.name = name
-        self.pitch = engine.pitch_of([self.field], nx)
-        self.op = engine.PointwiseOp(ny=ny, nx=nx, shift=shift, nan_to_zero=nan_to_zero, poly=poly,
+        self.op = engine.PointwiseOp(ny=self.ny, nx=self.nx, shift=shift, nan_to_zero=nan_to_zero, poly=poly,
                                      cell_scale=cell_scale, pitch=self.pitch)
-
-    def reduce(self, plan):
-        return self.op.reduce(plan, self.field)
-
-    def cells(self, timesum=False):
-        f = self._device_fields({"f": self.field})
-        return self.op.cells(f["f"], timesum=timesum)
 
 
 def _temperature_spec(ds):
@@ -322,34 +321,19 @@ class _CspSpec(_Spec):
     units = "kWh/kW_ref"
 
     def __init__(self, ds, installation):
-        ny, nx = _grid_shape(ds)
-        self.time_labels = pd.DatetimeIndex(_coord(ds, "time"))
+        super().__init__(ds)
         tech = installation["technology"]
         if tech not in _lib.CSP_TECH:
             raise ValueError(f'Unknown CSP technology option "{tech}".')
-        names = ["influx_direct"]
-        if _has(ds, "solar_azimuth") and _has(ds, "solar_altitude"):
-            dt = np.dtype(str(_raw(ds, "solar_altitude").dtype).replace("torch.", ""))
-            solar_src = _lib.SOLAR_STORED_F64 if dt == np.float64 else _lib.SOLAR_STORED_F32
-            names += ["solar_altitude", "solar_azimuth"]
-        else:
-            warnings.warn(_SOLAR_WARNING, DeprecationWarning)
-            solar_src = _lib.SOLAR_COMPUTED
+        solar_src, solar_names = _solar_source(ds)
         eff = EfficiencyTable.from_any(installation["efficiency"])
-        self.fields = {n: _raw(ds, n) for n in names}
-        self.pitch = engine.pitch_of(self.fields.values(), nx)
+        self._set_fields({n: _raw(ds, n) for n in ["influx_direct"] + solar_names})
         self.op = engine.CspOp(
-            ny=ny, nx=nx, time=self.time_labels, lon=_coord(ds, "lon").astype(np.float64),
+            ny=self.ny, nx=self.nx, time=self.time_labels, lon=_coord(ds, "lon").astype(np.float64),
             lat=_coord(ds, "lat").astype(np.float64), solar_src=solar_src,
             technology=_lib.CSP_TECH[tech], r_irradiance=installation["r_irradiance"],
             altitude=eff.altitude, azimuth=eff.azimuth, efficiency=eff.values, pitch=self.pitch,
         )
-
-    def reduce(self, plan):
-        return self.op.reduce(plan, self.fields)
-
-    def cells(self, timesum=False):
-        return self.op.cells(self._device_fields(self.fields), timesum=timesum)
 
 
 class _WindSpec(_Spec):
@@ -357,8 +341,7 @@ class _WindSpec(_Spec):
     units = "MWh/MWp"
 
     def __init__(self, ds, turbine, interpolation_method="logarithmic"):
-        ny, nx = _grid_shape(ds)
-        self.time_labels = pd.DatetimeIndex(_coord(ds, "time"))
+        super().__init__(ds)
         V, POW, hub_height, P = (turbine[k] for k in ("V", "POW", "hub_height", "P"))
         to_name = f"wnd{int(hub_height):0d}m"
         aux = None
@@ -392,18 +375,14 @@ class _WindSpec(_Spec):
                     f"Interpolation method must be 'logarithmic' or 'power',  but is: {interpolation_method}"
                 )
         self.wnd, self.aux = wnd, aux
-        self.pitch = engine.pitch_of([wnd, aux], nx)
+        self._set_fields({"wnd": wnd, "aux": aux})
         self.op = engine.WindOp(
-            ny=ny, nx=nx, V=np.asarray(V, float), POW_norm=np.asarray(POW, float) / P,
+            ny=self.ny, nx=self.nx, V=np.asarray(V, float), POW_norm=np.asarray(POW, float) / P,
             method=method, from_height=from_height, to_height=hub_height, pitch=self.pitch,
         )
 
     def reduce(self, plan):
         return self.op.reduce(plan, self.wnd, self.aux)
-
-    def cells(self, timesum=False):
-        f = self._device_fields({"wnd": self.wnd, "aux": self.aux})
-        return self.op.cells(f["wnd"], f["aux"], timesum=timesum)
 
 
 def day_bins(time, hour_shift):
@@ -426,19 +405,18 @@ class _HeatSpec(_Spec):
     cooling = False
 
     def __init__(self, ds, threshold, a, constant, hour_shift):
-        ny, nx = _grid_shape(ds)
+        super().__init__(ds)
         self.temp = _raw(ds, "temperature")
         self.time_labels, self.day_start = day_bins(_coord(ds, "time"), hour_shift)
-        self.pitch = engine.pitch_of([self.temp], nx)
-        self.op = engine.HeatOp(ny=ny, nx=nx, threshold=threshold, a=a, constant=constant,
+        self._set_fields({"temperature": self.temp})
+        self.op = engine.HeatOp(ny=self.ny, nx=self.nx, threshold=threshold, a=a, constant=constant,
                                 cooling=self.cooling, pitch=self.pitch)
 
     def reduce(self, plan):
         return self.op.reduce(plan, self.temp, self.day_start)
 
     def cells(self, timesum=False):
-        f = self._device_fields({"t": self.temp})
-        return self.op.cells(f["t"], self.day_start, timesum=timesum)
+        return self.op.cells(self._device_fields(), self.day_start, timesum=timesum)
 
 
 class _CoolingSpec(_HeatSpec):
@@ -628,11 +606,10 @@ def _partition(ds, n_time, devices, lazy, day_offsets=None):
                 cuts.append(c)
             if hi > cuts[-1]:
                 cuts.append(hi)
-        owner_of = lambda lo: next(devices[r] for r, (a, b) in enumerate(per_dev) if a <= lo < b)  # noqa: E731
     else:
         per_dev = [shard_bounds(n_time, n_dev, r) for r in range(n_dev)]
         cuts += [hi for lo, hi in per_dev if hi > lo]
-        owner_of = lambda lo: next(devices[r] for r, (a, b) in enumerate(per_dev) if a <= lo < b)  # noqa: E731
+    owner_of = lambda lo: next(devices[r] for r, (a, b) in enumerate(per_dev) if a <= lo < b)  # noqa: E731
     if day_offsets is not None:  # snap to day starts (first step of a day of the shifted axis)
         offs = np.asarray(day_offsets)
         snapped = sorted({int(offs[np.argmin(np.abs(offs - c))]) for c in cuts[1:-1]} | {0, n_time})
@@ -758,32 +735,9 @@ def _layout_values(layout, ds):
     return out.reshape(-1)
 
 
-def convert_and_aggregate(
-    cutout,
-    convert_func,
-    matrix=None,
-    index=None,
-    layout=None,
-    shapes=None,
-    shapes_crs=4326,
-    per_unit=False,
-    return_capacity=False,
-    aggregate_time="legacy",
-    capacity_factor=False,
-    capacity_factor_timeseries=False,
-    show_progress=False,
-    dask_kwargs={},
-    **convert_kwds,
-):
-    """Convert and aggregate a weather-based renewable generation time-series.
-
-    Same contract as the reference (convert.py:59-276): ``matrix`` (N x S, in
-    ``cutout.grid`` order), ``shapes`` or ``layout`` select spatial
-    aggregation; ``per_unit`` / ``return_capacity``; ``aggregate_time`` in
-    {"sum", "mean", "legacy", None}; deprecated ``capacity_factor*`` flags.
-    ``show_progress`` and ``dask_kwargs`` are accepted and ignored (the result
-    is computed eagerly on the GPU and returned loaded).
-    """
+def _aggregate_time_arg(aggregate_time, capacity_factor, capacity_factor_timeseries):
+    """``aggregate_time`` after the deprecated ``capacity_factor*`` flags (convert.py:183-217);
+    the warnings point at the caller of ``convert_and_aggregate``."""
     if aggregate_time not in ("sum", "mean", "legacy", None):
         raise ValueError(
             f"aggregate_time must be 'sum', 'mean', 'legacy', or None, got {aggregate_time!r}"
@@ -793,7 +747,7 @@ def convert_and_aggregate(
             "aggregate_time='legacy' is deprecated and will be removed in a "
             "future release. Pass 'sum', 'mean', or None explicitly.",
             FutureWarning,
-            stacklevel=2,
+            stacklevel=3,
         )
     if capacity_factor or capacity_factor_timeseries:
         if aggregate_time != "legacy":
@@ -805,102 +759,22 @@ def convert_and_aggregate(
             warnings.warn(
                 "capacity_factor is deprecated. Use aggregate_time='mean' instead.",
                 FutureWarning,
-                stacklevel=2,
+                stacklevel=3,
             )
             aggregate_time = "mean"
         if capacity_factor_timeseries:
             warnings.warn(
                 "capacity_factor_timeseries is deprecated. Use aggregate_time=None instead.",
                 FutureWarning,
-                stacklevel=2,
+                stacklevel=3,
             )
             aggregate_time = None
+    return aggregate_time
 
-    func_name = convert_func.__name__.replace("convert_", "")
-    logger.info(f"Convert and aggregate '{func_name}'.")
-    ds = cutout.data
-    ny, nx = _grid_shape(ds)
-    spec_cls = _known_spec(convert_func)
-    shard = getattr(cutout, "time_shard", None)  # multi-GPU time sharding (dist.py)
-    devices = list(getattr(cutout, "devices", None) or [])
-    lazy = _is_dask_backed(ds)
-    # several GPUs from this one process, and/or a lazily loaded (dask-backed) cutout that
-    # is converted time part by time part instead of being materialised whole
-    partitioned = spec_cls is not None and (len(devices) > 1 or lazy) and _is_host_resident(ds)
-    if partitioned and shard is not None:
-        raise ValueError("a cutout is either time-sharded across processes (time_shard=) or fanned "
-                         "out to several devices by one process (devices=), not both")
-    if len(devices) == 1 and not partitioned:
-        engine._torch().cuda.set_device(devices[0])
-    if partitioned:
-        spec, da = None, None
-    elif spec_cls is not None:
-        spec, da = spec_cls(ds, **convert_kwds), None
-    else:  # plugin protocol: the callable produces the (time, y, x) field itself
-        spec, da = None, convert_func(ds, **convert_kwds)
 
-    if partitioned:
-        n_time = len(_coord(ds, "time"))
-        day_offsets = None
-        if spec_cls in (_HeatSpec, _CoolingSpec):
-            day_offsets = day_bins(_coord(ds, "time"), convert_kwds.get("hour_shift", 0.0))[1]
-        parts = _partition(ds, n_time, devices or [engine.current_device()], lazy, day_offsets)
-        wpd = 2 if lazy else 1
-    no_args = all(v is None for v in [layout, shapes, matrix])
-
-    if no_args:
-        if per_unit or return_capacity:
-            raise ValueError(
-                "One of `matrix`, `shapes` and `layout` must be "
-                "given for `per_unit` or `return_capacity`"
-            )
-        agg = "sum" if aggregate_time == "legacy" else aggregate_time
-        if partitioned:
-            coords_yx = {"y": _coord(ds, "y"), "x": _coord(ds, "x")}
-            if agg is None:
-                res = _run_partitioned(ds, spec_cls, convert_kwds, parts,
-                                       lambda sp_, dev: _to_host(sp_.cells()), wpd)
-                sp0 = res[0][1]
-                attrs = {"units": sp0.units} if sp0.units else {}
-                labels = pd.Index(np.concatenate([np.asarray(sp_.time_labels) for _, sp_ in res]))
-                vals = np.concatenate([v for v, _ in res], axis=0)
-                return make_dataarray(vals, ("time", "y", "x"), {"time": labels, **coords_yx}, attrs, sp0.name)
-            res = _run_partitioned(ds, spec_cls, convert_kwds, parts,
-                                   lambda sp_, dev: tuple(_to_host(a).astype(np.float64) for a in sp_.cells_timesum()), wpd)
-            sp0 = res[0][1]
-            attrs = {"units": sp0.units} if sp0.units else {}
-            total = sum(v[0] for v, _ in res)
-            count = sum(v[1] for v, _ in res)
-            if agg == "mean":
-                with np.errstate(divide="ignore", invalid="ignore"):
-                    total = np.where(count > 0, total / count, np.nan)
-            return make_dataarray(total, ("y", "x"), coords_yx, attrs, sp0.name)
-        if spec is None:
-            if agg == "sum":
-                return da.sum("time", keep_attrs=True)
-            if agg == "mean":
-                return da.mean("time", keep_attrs=True)
-            return da
-        coords_yx = {"y": _coord(ds, "y"), "x": _coord(ds, "x")}
-        attrs = {"units": spec.units} if spec.units else {}
-        if agg is None:
-            vals = _to_host(spec.cells())
-            labels = spec.time_labels
-            if shard is not None:
-                vals, labels = shard.gather_time(vals, labels)
-            return make_dataarray(vals, ("time", "y", "x"), {"time": labels, **coords_yx}, attrs, spec.name)
-        # NaN-skipping time sum and the number of valid steps per cell (da.sum / da.mean
-        # over "time" skip NaN, convert.py:51-56; an all-NaN cell has mean NaN, sum 0)
-        total, count = spec.cells_timesum()
-        if shard is not None:
-            total, count = shard.sum_planes(total, count)
-        vals = _to_host(total).astype(np.float64)
-        if agg == "mean":
-            cnt = _to_host(count).astype(np.float64)
-            with np.errstate(divide="ignore", invalid="ignore"):
-                vals = np.where(cnt > 0, vals / cnt, np.nan)
-        return make_dataarray(vals, ("y", "x"), coords_yx, attrs, spec.name)
-
+def _aggregation_matrix(cutout, ds, matrix, index, layout, shapes, shapes_crs):
+    """``matrix`` / ``shapes`` / ``layout`` / ``index`` -> (CSR aggregation matrix, bus dim name,
+    bus index) (convert.py:233-255)."""
     if matrix is not None:
         if shapes is not None:
             raise ValueError("Passing matrix and shapes is ambiguous. Pass only one of them.")
@@ -936,37 +810,146 @@ def convert_and_aggregate(
 
     assert isinstance(matrix, sp.csr_matrix)
     dim, idx = _ensure_index(index, matrix.shape[0])
+    return matrix, dim, idx
 
+
+class _PluginSpec:
+    """A plugin's (time, y, x) result on the reduce path: only the aggregation runs on the GPU
+    (``atl_spmm``).  A result computed from a row-padded device cutout keeps the padding."""
+
+    def __init__(self, da):
+        self.da = da
+        self.values = da if engine._is_torch(da) else getattr(da, "values", da)
+        self.pitch = int(self.values.shape[-1]) if engine._is_torch(self.values) and self.values.ndim == 3 else None
+        self.name = getattr(da, "name", None)
+
+    def reduce(self, plan):
+        return plan.spmm(self.values if engine._is_torch(self.values) else np.asarray(self.values))
+
+    @property
+    def time_labels(self):
+        if hasattr(self.da, "coords"):
+            return pd.Index(np.asarray(self.da.coords["time"]))
+        return pd.RangeIndex(len(self.values))
+
+
+def _joined(res):
+    """Per-part [(values, labels)] -> (values, time labels) joined along time."""
+    if len(res) == 1:
+        return res[0][0], res[0][1].time_labels
+    labels = pd.Index(np.concatenate([np.asarray(m.time_labels) for _, m in res]))
+    if isinstance(res[0][1].time_labels, pd.DatetimeIndex):
+        labels = pd.DatetimeIndex(labels)
+    return np.concatenate([v for v, _ in res], axis=0), labels
+
+
+def convert_and_aggregate(
+    cutout,
+    convert_func,
+    matrix=None,
+    index=None,
+    layout=None,
+    shapes=None,
+    shapes_crs=4326,
+    per_unit=False,
+    return_capacity=False,
+    aggregate_time="legacy",
+    capacity_factor=False,
+    capacity_factor_timeseries=False,
+    show_progress=False,
+    dask_kwargs={},
+    **convert_kwds,
+):
+    """Convert and aggregate a weather-based renewable generation time-series.
+
+    Same contract as the reference (convert.py:59-276): ``matrix`` (N x S, in
+    ``cutout.grid`` order), ``shapes`` or ``layout`` select spatial
+    aggregation; ``per_unit`` / ``return_capacity``; ``aggregate_time`` in
+    {"sum", "mean", "legacy", None}; deprecated ``capacity_factor*`` flags.
+    ``show_progress`` and ``dask_kwargs`` are accepted and ignored (the result
+    is computed eagerly on the GPU and returned loaded).
+    """
+    aggregate_time = _aggregate_time_arg(aggregate_time, capacity_factor, capacity_factor_timeseries)
+    func_name = convert_func.__name__.replace("convert_", "")
+    logger.info(f"Convert and aggregate '{func_name}'.")
+    ds = cutout.data
+    ny, nx = _grid_shape(ds)
+    spec_cls = _known_spec(convert_func)
+    shard = getattr(cutout, "time_shard", None)  # multi-GPU time sharding (dist.py)
+    devices = list(getattr(cutout, "devices", None) or [])
+    lazy = _is_dask_backed(ds)
+    # several GPUs from this one process, and/or a lazily loaded (dask-backed) cutout that
+    # is converted time part by time part instead of being materialised whole
+    partitioned = spec_cls is not None and (len(devices) > 1 or lazy) and _is_host_resident(ds)
+    if partitioned and shard is not None:
+        raise ValueError("a cutout is either time-sharded across processes (time_shard=) or fanned "
+                         "out to several devices by one process (devices=), not both")
+    spec = da = parts = None
     if partitioned:
-        digest = engine.matrix_digest(matrix)
-        res = _run_partitioned(
-            ds, spec_cls, convert_kwds, parts,
-            lambda sp_, dev: _to_host(sp_.reduce(engine.get_plan(matrix, ny, nx, device=dev, pitch=sp_.pitch,
-                                                                 digest=digest))), wpd)
-        time_labels = pd.Index(np.concatenate([np.asarray(sp_.time_labels) for _, sp_ in res]))
-        if isinstance(res[0][1].time_labels, pd.DatetimeIndex):
-            time_labels = pd.DatetimeIndex(time_labels)
-        name = res[0][1].name
-        res = np.concatenate([v for v, _ in res], axis=0)
-    pitch = getattr(spec, "pitch", None)
-    if partitioned:
-        pass
-    elif spec is None:  # plugin result computed from a row-padded device cutout keeps the padding
-        vals0 = da if engine._is_torch(da) else getattr(da, "values", da)
-        if engine._is_torch(vals0) and vals0.ndim == 3 and vals0.shape[-1] != nx:
-            pitch = int(vals0.shape[-1])
-    if not partitioned:
-        plan = engine.get_plan(matrix, ny, nx, pitch=pitch)
-    if partitioned:
-        pass
-    elif spec is not None:
-        res = spec.reduce(plan)  # (time, bus) float32
-        time_labels, name = spec.time_labels, spec.name
+        day_offsets = None
+        if spec_cls in (_HeatSpec, _CoolingSpec):
+            day_offsets = day_bins(_coord(ds, "time"), convert_kwds.get("hour_shift", 0.0))[1]
+        parts = _partition(ds, len(_coord(ds, "time")), devices or [engine.current_device()], lazy, day_offsets)
     else:
-        vals = da if engine._is_torch(da) else getattr(da, "values", da)
-        res = plan.spmm(np.asarray(vals) if not engine._is_torch(vals) else vals)
-        time_labels = pd.Index(np.asarray(da.coords["time"])) if hasattr(da, "coords") else pd.RangeIndex(len(vals))
-        name = getattr(da, "name", None)
+        if len(devices) == 1:
+            engine._torch().cuda.set_device(devices[0])
+        if spec_cls is not None:
+            spec = spec_cls(ds, **convert_kwds)
+        else:  # plugin protocol: the callable produces the (time, y, x) field itself
+            da = convert_func(ds, **convert_kwds)
+
+    def execute(spec, run):
+        """[(result, labels)] of ``run(spec, device)`` per time part.  In-process: ``spec`` on
+        the caller's thread, its result left where it was computed; partitioned: a spec per
+        part on its device, its result moved to the host."""
+        if parts is None:
+            return [(run(spec, None), spec)]
+        return _run_partitioned(ds, spec_cls, convert_kwds, parts, lambda sp_, dev: _to_host(run(sp_, dev)),
+                                2 if lazy else 1)
+
+    if all(v is None for v in [layout, shapes, matrix]):
+        if per_unit or return_capacity:
+            raise ValueError(
+                "One of `matrix`, `shapes` and `layout` must be "
+                "given for `per_unit` or `return_capacity`"
+            )
+        agg = "sum" if aggregate_time == "legacy" else aggregate_time
+        if da is not None:
+            if agg == "sum":
+                return da.sum("time", keep_attrs=True)
+            if agg == "mean":
+                return da.mean("time", keep_attrs=True)
+            return da
+        res = execute(spec, lambda sp_, dev: sp_.cells(timesum=agg is not None))
+        meta = res[0][1]
+        coords_yx = {"y": _coord(ds, "y"), "x": _coord(ds, "x")}
+        attrs = {"units": meta.units} if meta.units else {}
+        if agg is None:
+            vals, labels = _joined(res)
+            vals = _to_host(vals)
+            if shard is not None:
+                vals, labels = shard.gather_time(vals, labels)
+            return make_dataarray(vals, ("time", "y", "x"), {"time": labels, **coords_yx}, attrs, meta.name)
+        # NaN-skipping time sum and the number of valid steps per cell (da.sum / da.mean
+        # over "time" skip NaN, convert.py:51-56; an all-NaN cell has mean NaN, sum 0)
+        planes = [(v[0], v[1]) for v, _ in res]
+        if shard is not None:
+            planes = [shard.sum_planes(*planes[0])]
+        total = sum(_to_host(t).astype(np.float64) for t, _ in planes)
+        if agg == "mean":
+            count = sum(_to_host(c).astype(np.float64) for _, c in planes)
+            with np.errstate(divide="ignore", invalid="ignore"):
+                total = np.where(count > 0, total / count, np.nan)
+        return make_dataarray(total, ("y", "x"), coords_yx, attrs, meta.name)
+
+    matrix, dim, idx = _aggregation_matrix(cutout, ds, matrix, index, layout, shapes, shapes_crs)
+    if da is not None:
+        spec = _PluginSpec(da)
+    digest = engine.matrix_digest(matrix)
+    res = execute(spec, lambda sp_, dev: sp_.reduce(engine.get_plan(matrix, ny, nx, device=dev, pitch=sp_.pitch,
+                                                              digest=digest)))  # (time, bus) float32
+    name = res[0][1].name
+    res, time_labels = _joined(res)
     if shard is not None:
         res, time_labels = shard.gather_time(res, time_labels)
     capacity = caps = None
@@ -978,7 +961,7 @@ def convert_and_aggregate(
     # dim order mirrors aggregate.py: (time, bus) for dask-backed cutouts
     # (:24-32), (bus, time) for NumPy-backed ones (:34-35)
     agg = aggregate_time if aggregate_time != "legacy" else None
-    bus_major = agg is None and not _is_dask_backed(ds)
+    bus_major = agg is None and not lazy
     results = _finish_results(res, caps if per_unit else None, agg, bus_major)
     if agg is not None:
         out = make_dataarray(results, (dim,), {dim: idx}, {"units": units}, name)

@@ -197,14 +197,36 @@ def get_plan(matrix, ny, nx, device=None, pitch=None, digest=None):
     return plan
 
 
+def _first(fields):
+    return next(a for a in fields.values() if a is not None)
+
+
 class _Op:
-    _destroy = None
+    """A fused operator, ``atl_<_name>_*`` of the C ABI.  A subclass declares its fields:
+    ``_struct`` is the ctypes struct of field pointers (None: one bare field pointer) and
+    ``_f64`` the fields that may be float64 (stored solar position).  ``_slab`` forms the
+    arguments that follow the fields in the C call."""
+
+    _name = None
+    _struct = None
+    _f64 = ()
+
+    def _bind(self, ny, nx, device, pitch):
+        _lib.load()
+        self.device = current_device() if device is None else device
+        self.ny, self.nx = ny, nx
+        self.pitch = int(pitch) or nx
+
+    def _create(self, cfg):
+        h = C.c_void_p()
+        _lib.check(getattr(_lib.load(), f"atl_{self._name}_create")(self.device, C.byref(cfg), C.byref(h)))
+        self.handle = h
 
     def __del__(self):
         h = getattr(self, "handle", None)
         if h:
             try:
-                getattr(_lib.load(), self._destroy)(h)
+                getattr(_lib.load(), f"atl_{self._name}_destroy")(h)
             except Exception:  # noqa: BLE001
                 pass
             self.handle = None
@@ -216,19 +238,14 @@ class _Op:
             raise ValueError("mixing host (NumPy) and device (torch) fields in one call")
         return kinds.pop() if kinds else False
 
-    def _out(self, shape, like):
-        torch = _torch()
-        return torch.empty(shape, dtype=torch.float32, device=like.device)
-
     def _dev(self, a, f64_ok=False):
         """Device field -> contiguous tensor, after checking what the kernels assume
         about it: (time, ny, pitch) layout on this operator's GPU, float32 (float64
         for stored solar position).  The C ABI takes raw pointers, so this is the
         only place a wrong shape can be caught."""
         torch = _torch()
-        pitch = getattr(self, "pitch", 0) or self.nx
-        if a.ndim != 3 or tuple(a.shape[1:]) != (self.ny, pitch):
-            raise ValueError(f"field has shape {tuple(a.shape)}, expected (time, {self.ny}, {pitch})")
+        if a.ndim != 3 or tuple(a.shape[1:]) != (self.ny, self.pitch):
+            raise ValueError(f"field has shape {tuple(a.shape)}, expected (time, {self.ny}, {self.pitch})")
         if a.dtype != torch.float32 and not (f64_ok and a.dtype == torch.float64):
             raise TypeError(f"device fields must be float32, got {a.dtype}")
         if a.device.type != "cuda" or a.device.index != self.device:
@@ -243,29 +260,76 @@ class _Op:
             return np.ascontiguousarray(a)
         return host_f32(a)
 
-    @staticmethod
-    def _empty_like(first, shape):
-        """Result for an empty time axis (e.g. a rank whose time shard is empty): no
-        kernel is launched (empty tensors have NULL data pointers)."""
-        if _is_torch(first):
-            torch = _torch()
-            return torch.zeros(shape, dtype=torch.float32, device=first.device)
-        return np.zeros(shape, dtype=np.float32)
+    def _pack(self, fields, dev):
+        """Checked fields -> (the C call's field argument, the arrays it points into)."""
+        check, ptr = (self._dev, _dptr) if dev else (self._host, _hptr)
+        names = list(fields) if self._struct is None else [n for n, _ in self._struct._fields_]
+        keep = {n: check(fields[n], f64_ok=n in self._f64) for n in names if fields.get(n) is not None}
+        if self._struct is None:
+            (a,) = keep.values()
+            return ptr(a), keep
+        f = self._struct()
+        for n in names:
+            setattr(f, n, ptr(keep[n]).value if n in keep else None)
+        return C.byref(f), keep
+
+    def _call(self, kind, fields, slab, n, plan=None, chunk=0):
+        """``atl_<op>_<kind>`` on ``fields`` (name -> (time, y, x) array or None), ``slab`` = the
+        arguments after the fields, ``n`` = output steps.  kind "reduce": (n, n_bus) float32,
+        a torch CUDA tensor for device fields, an ndarray for host fields (``*_reduce_host``
+        streams them in slabs of ``chunk``); "cells": (n, ny, nx); "timesum": (2, ny, nx) =
+        NaN-skipping sum | valid steps.  Per-cell outputs take device fields only."""
+        dev = self._all_device(fields.values()) if kind == "reduce" else True
+        first = _first(fields)
+        shape = (2, self.ny, self.nx) if kind == "timesum" else \
+            (n, plan.n_bus) if kind == "reduce" else (n, self.ny, self.nx)
+        if n == 0 or first.shape[0] == 0:
+            # e.g. a rank whose time shard is empty: no kernel is launched (empty tensors
+            # have NULL data pointers)
+            if _is_torch(first):
+                torch = _torch()
+                return torch.zeros(shape, dtype=torch.float32, device=first.device)
+            return np.zeros(shape, dtype=np.float32)
+        arg, keep = self._pack(fields, dev)
+        head = (self.handle, plan.handle) if kind == "reduce" else (self.handle,)
+        if not dev:
+            out = np.empty(shape, dtype=np.float32)
+            _lib.check(getattr(_lib.load(), f"atl_{self._name}_reduce_host")(*head, arg, *slab, _hptr(out), chunk))
+            return out
+        torch = _torch()
+        if kind == "timesum":
+            out = torch.zeros(shape, dtype=torch.float32, device=first.device)
+            outs = (_dptr(out[0]), _dptr(out[1]))
+        else:
+            out = torch.empty(shape, dtype=torch.float32, device=first.device)
+            outs = (_dptr(out),)
+        _lib.check(getattr(_lib.load(), f"atl_{self._name}_{kind}")(*head, arg, *slab, *outs, _stream_ptr()))
+        return out
+
+    def _slab(self, fields):
+        """(the C call's arguments after the fields, output steps) for whole fields."""
+        nt = _first(fields).shape[0]
+        return (nt,), nt
+
+    def reduce(self, plan, fields, chunk_steps=0):
+        slab, n = self._slab(fields)
+        return self._call("reduce", fields, slab, n, plan, chunk_steps)
+
+    def cells(self, fields, timesum=False):
+        """Per-cell values (nt, ny, nx) or their time sum (2, ny, nx); device fields only."""
+        slab, n = self._slab(fields)
+        return self._call("timesum" if timesum else "cells", fields, slab, n)
 
 
 class PvOp(_Op):
     """convert_pv (convert.py:840-854) operator; see include/atlite_b200.h."""
 
-    _destroy = "atl_pv_destroy"
-    FIELD_NAMES = tuple(n for n, _ in _lib.PvFields._fields_)
+    _name, _struct, _f64 = "pv", _lib.PvFields, ("solar_altitude", "solar_azimuth")
 
     def __init__(self, *, ny, nx, time, lon, lat, slope, azimuth, tracking, trigon_model,
                  clearsky_model, irr_branch, albedo_src, solar_src, panel=None, time_shift="0h",
                  altitude_threshold=1.0, output="panel", thermal=(0.0, 0.0, 0.0), device=None, pitch=0):
-        lib = _lib.load()
-        self.device = current_device() if device is None else device
-        self.ny, self.nx = ny, nx
-        self.pitch = int(pitch) or nx
+        self._bind(ny, nx, device, pitch)
         self._time = time_ns(time)
         self.nt = len(self._time)
         self._lon, self._lat = _lib.as_f64(lon), _lib.as_f64(lat)
@@ -306,73 +370,25 @@ class PvOp(_Op):
             vals += [panel.get("inverter_efficiency", 1.0)]
         for i, v in enumerate(vals):
             cfg.panel[i] = float(v)
-        h = C.c_void_p()
-        _lib.check(lib.atl_pv_create(self.device, C.byref(cfg), C.byref(h)))
-        self.handle = h
-
-    def _fields(self, fields, host):
-        f = _lib.PvFields()
-        keep = []
-        for n in self.FIELD_NAMES:
-            a = fields.get(n)
-            if a is None:
-                setattr(f, n, None)
-                continue
-            if host:
-                a = self._host(a, f64_ok=n.startswith("solar_"))
-                keep.append(a)
-                setattr(f, n, a.ctypes.data)
-            else:
-                a = self._dev(a, f64_ok=n.startswith("solar_"))
-                keep.append(a)
-                setattr(f, n, a.data_ptr())
-        return f, keep
+        self._create(cfg)
 
     def reduce(self, plan, fields, t0=0, nt=None, chunk_steps=0):
         """(nt, n_bus) float32: torch CUDA tensor for device fields, ndarray for host fields."""
-        lib = _lib.load()
-        dev = self._all_device(fields.values())
-        first = next(a for a in fields.values() if a is not None)
-        nt = first.shape[0] if nt is None else nt
-        if nt == 0:
-            return self._empty_like(first, (0, plan.n_bus))
-        f, keep = self._fields(fields, host=not dev)
-        if dev:
-            out = self._out((nt, plan.n_bus), first)
-            _lib.check(lib.atl_pv_reduce(self.handle, plan.handle, C.byref(f), t0, nt, _dptr(out), _stream_ptr()))
-            return out
-        out = np.empty((nt, plan.n_bus), dtype=np.float32)
-        _lib.check(lib.atl_pv_reduce_host(self.handle, plan.handle, C.byref(f), t0, nt, _hptr(out), chunk_steps))
-        return out
+        nt = _first(fields).shape[0] if nt is None else nt
+        return self._call("reduce", fields, (t0, nt), nt, plan, chunk_steps)
 
-    def cells(self, fields, t0=0, timesum=False):
-        """Per-cell values (nt, ny, nx) or their time sum (ny, nx); device fields only."""
-        lib = _lib.load()
-        first = next(a for a in fields.values() if a is not None)
-        nt = first.shape[0]
-        if nt == 0:
-            return self._empty_like(first, (2, self.ny, self.nx) if timesum else (0, self.ny, self.nx))
-        f, keep = self._fields(fields, host=False)
-        torch = _torch()
-        if timesum:
-            out = torch.zeros((2, self.ny, self.nx), dtype=torch.float32, device=first.device)  # sum | valid steps
-            _lib.check(lib.atl_pv_timesum(self.handle, C.byref(f), t0, nt, _dptr(out[0]), _dptr(out[1]), _stream_ptr()))
-        else:
-            out = self._out((nt, self.ny, self.nx), first)
-            _lib.check(lib.atl_pv_cells(self.handle, C.byref(f), t0, nt, _dptr(out), _stream_ptr()))
-        return out
+    def _slab(self, fields):
+        nt = _first(fields).shape[0]
+        return (0, nt), nt
 
 
 class WindOp(_Op):
     """convert_wind (convert.py:634-662) operator."""
 
-    _destroy = "atl_wind_destroy"
+    _name, _struct = "wind", _lib.WindFields
 
     def __init__(self, *, ny, nx, V, POW_norm, method, from_height, to_height, device=None, pitch=0):
-        lib = _lib.load()
-        self.device = current_device() if device is None else device
-        self.ny, self.nx = ny, nx
-        self.pitch = int(pitch) or nx
+        self._bind(ny, nx, device, pitch)
         self._V, self._P = _lib.as_f64(V), _lib.as_f64(POW_norm)
         cfg = _lib.WindConfig()
         cfg.ny, cfg.nx, cfg.method = ny, nx, method
@@ -380,120 +396,44 @@ class WindOp(_Op):
         cfg.pitch = int(pitch)
         cfg.n_knots = len(self._V)
         cfg.V, cfg.POW_norm = _lib.ptr(self._V).value, _lib.ptr(self._P).value
-        h = C.c_void_p()
-        _lib.check(lib.atl_wind_create(self.device, C.byref(cfg), C.byref(h)))
-        self.handle = h
-
-    def _fields(self, wnd, aux, host):
-        f = _lib.WindFields()
-        keep = []
-        for n, a in (("wnd", wnd), ("aux", aux)):
-            if a is None:
-                setattr(f, n, None)
-            elif host:
-                a = self._host(a)
-                keep.append(a)
-                setattr(f, n, a.ctypes.data)
-            else:
-                a = self._dev(a)
-                keep.append(a)
-                setattr(f, n, a.data_ptr())
-        return f, keep
+        self._create(cfg)
 
     def reduce(self, plan, wnd, aux=None, chunk_steps=0):
-        lib = _lib.load()
-        dev = self._all_device([wnd, aux])
-        nt = wnd.shape[0]
-        if nt == 0:
-            return self._empty_like(wnd, (0, plan.n_bus))
-        f, keep = self._fields(wnd, aux, host=not dev)
-        if dev:
-            out = self._out((nt, plan.n_bus), wnd)
-            _lib.check(lib.atl_wind_reduce(self.handle, plan.handle, C.byref(f), nt, _dptr(out), _stream_ptr()))
-            return out
-        out = np.empty((nt, plan.n_bus), dtype=np.float32)
-        _lib.check(lib.atl_wind_reduce_host(self.handle, plan.handle, C.byref(f), nt, _hptr(out), chunk_steps))
-        return out
-
-    def cells(self, wnd, aux=None, timesum=False):
-        lib = _lib.load()
-        nt = wnd.shape[0]
-        if nt == 0:
-            return self._empty_like(wnd, (2, self.ny, self.nx) if timesum else (0, self.ny, self.nx))
-        f, keep = self._fields(wnd, aux, host=False)
-        torch = _torch()
-        if timesum:
-            out = torch.zeros((2, self.ny, self.nx), dtype=torch.float32, device=wnd.device)
-            _lib.check(lib.atl_wind_timesum(self.handle, C.byref(f), nt, _dptr(out[0]), _dptr(out[1]), _stream_ptr()))
-        else:
-            out = self._out((nt, self.ny, self.nx), wnd)
-            _lib.check(lib.atl_wind_cells(self.handle, C.byref(f), nt, _dptr(out), _stream_ptr()))
-        return out
+        return super().reduce(plan, {"wnd": wnd, "aux": aux}, chunk_steps)
 
 
 class HeatOp(_Op):
     """convert_heat_demand (convert.py:405-418) operator."""
 
-    _destroy = "atl_heat_destroy"
+    _name = "heat"
 
     def __init__(self, *, ny, nx, threshold, a, constant, cooling=False, device=None, pitch=0):
-        lib = _lib.load()
-        self.device = current_device() if device is None else device
-        self.ny, self.nx = ny, nx
-        self.pitch = int(pitch) or nx
+        self._bind(ny, nx, device, pitch)
         cfg = _lib.HeatConfig()
         cfg.ny, cfg.nx = ny, nx
         cfg.threshold_c, cfg.a, cfg.constant = float(threshold), float(a), float(constant)
         cfg.cooling = 1 if cooling else 0
         cfg.pitch = int(pitch)
-        h = C.c_void_p()
-        _lib.check(lib.atl_heat_create(self.device, C.byref(cfg), C.byref(h)))
-        self.handle = h
+        self._create(cfg)
 
     def reduce(self, plan, temperature, day_start, chunk_days=0):
-        lib = _lib.load()
         ds = np.ascontiguousarray(day_start, dtype=np.int64)
-        nd = len(ds) - 1
-        if nd == 0 or temperature.shape[0] == 0:
-            return self._empty_like(temperature, (nd, plan.n_bus))
-        if _is_torch(temperature):
-            t = self._dev(temperature)
-            out = self._out((nd, plan.n_bus), t)
-            _lib.check(lib.atl_heat_reduce(self.handle, plan.handle, _dptr(t), _lib.ptr(ds), nd, _dptr(out), _stream_ptr()))
-            return out
-        t = self._host(temperature)
-        out = np.empty((nd, plan.n_bus), dtype=np.float32)
-        _lib.check(lib.atl_heat_reduce_host(self.handle, plan.handle, _hptr(t), _lib.ptr(ds), nd, _hptr(out), chunk_days))
-        return out
+        return self._call("reduce", {"temperature": temperature}, (_lib.ptr(ds), len(ds) - 1), len(ds) - 1,
+                          plan, chunk_days)
 
-    def cells(self, temperature, day_start, timesum=False):
-        lib = _lib.load()
+    def cells(self, fields, day_start, timesum=False):
         ds = np.ascontiguousarray(day_start, dtype=np.int64)
-        nd = len(ds) - 1
-        if nd == 0 or temperature.shape[0] == 0:
-            return self._empty_like(temperature, (2, self.ny, self.nx) if timesum else (nd, self.ny, self.nx))
-        t = self._dev(temperature)
-        torch = _torch()
-        if timesum:
-            out = torch.zeros((2, self.ny, self.nx), dtype=torch.float32, device=t.device)
-            _lib.check(lib.atl_heat_timesum(self.handle, _dptr(t), _lib.ptr(ds), nd, _dptr(out[0]), _dptr(out[1]), _stream_ptr()))
-        else:
-            out = self._out((nd, self.ny, self.nx), t)
-            _lib.check(lib.atl_heat_cells(self.handle, _dptr(t), _lib.ptr(ds), nd, _dptr(out), _stream_ptr()))
-        return out
+        return self._call("timesum" if timesum else "cells", fields, (_lib.ptr(ds), len(ds) - 1), len(ds) - 1)
 
 
 class PointwiseOp(_Op):
     """Pointwise function of one field (temperature family, COP, runoff x height);
     see include/atlite_b200.h."""
 
-    _destroy = "atl_pointwise_destroy"
+    _name = "pointwise"
 
     def __init__(self, *, ny, nx, shift=0.0, nan_to_zero=False, poly=None, cell_scale=None, device=None, pitch=0):
-        lib = _lib.load()
-        self.device = current_device() if device is None else device
-        self.ny, self.nx = ny, nx
-        self.pitch = int(pitch) or nx
+        self._bind(ny, nx, device, pitch)
         cfg = _lib.PointwiseConfig()
         cfg.ny, cfg.nx = ny, nx
         cfg.shift = float(shift)
@@ -508,52 +448,17 @@ class PointwiseOp(_Op):
             if self._scale.shape != (ny, nx):
                 raise ValueError(f"cell_scale must have shape {(ny, nx)}, has {self._scale.shape}")
             cfg.cell_scale = self._scale.ctypes.data
-        h = C.c_void_p()
-        _lib.check(lib.atl_pointwise_create(self.device, C.byref(cfg), C.byref(h)))
-        self.handle = h
-
-    def reduce(self, plan, field, chunk_steps=0):
-        lib = _lib.load()
-        nt = field.shape[0]
-        if nt == 0:
-            return self._empty_like(field, (0, plan.n_bus))
-        if _is_torch(field):
-            f = self._dev(field)
-            out = self._out((nt, plan.n_bus), f)
-            _lib.check(lib.atl_pointwise_reduce(self.handle, plan.handle, _dptr(f), nt, _dptr(out), _stream_ptr()))
-            return out
-        f = self._host(field)
-        out = np.empty((nt, plan.n_bus), dtype=np.float32)
-        _lib.check(lib.atl_pointwise_reduce_host(self.handle, plan.handle, _hptr(f), nt, _hptr(out), chunk_steps))
-        return out
-
-    def cells(self, field, timesum=False):
-        lib = _lib.load()
-        nt = field.shape[0]
-        if nt == 0:
-            return self._empty_like(field, (2, self.ny, self.nx) if timesum else (0, self.ny, self.nx))
-        f = self._dev(field)
-        torch = _torch()
-        if timesum:
-            out = torch.zeros((2, self.ny, self.nx), dtype=torch.float32, device=f.device)
-            _lib.check(lib.atl_pointwise_timesum(self.handle, _dptr(f), nt, _dptr(out[0]), _dptr(out[1]), _stream_ptr()))
-        else:
-            out = self._out((nt, self.ny, self.nx), f)
-            _lib.check(lib.atl_pointwise_cells(self.handle, _dptr(f), nt, _dptr(out), _stream_ptr()))
-        return out
+        self._create(cfg)
 
 
 class CspOp(_Op):
     """convert_csp (convert.py:940-972) operator."""
 
-    _destroy = "atl_csp_destroy"
+    _name, _struct, _f64 = "csp", _lib.CspFields, ("solar_altitude", "solar_azimuth")
 
     def __init__(self, *, ny, nx, time, lon, lat, solar_src, technology, r_irradiance, altitude, azimuth,
                  efficiency, time_shift="0h", dni_altitude_threshold=3.75, device=None, pitch=0):
-        lib = _lib.load()
-        self.device = current_device() if device is None else device
-        self.ny, self.nx = ny, nx
-        self.pitch = int(pitch) or nx
+        self._bind(ny, nx, device, pitch)
         self._time = time_ns(time)
         self._lon, self._lat = _lib.as_f64(lon), _lib.as_f64(lat)
         self._alt, self._az, self._eff = _lib.as_f64(altitude), _lib.as_f64(azimuth), _lib.as_f64(efficiency)
@@ -570,55 +475,6 @@ class CspOp(_Op):
         cfg.n_alt, cfg.n_az = len(self._alt), len(self._az)
         cfg.altitude_rad, cfg.azimuth_rad = _lib.ptr(self._alt).value, _lib.ptr(self._az).value
         cfg.efficiency = _lib.ptr(self._eff).value
-        h = C.c_void_p()
-        _lib.check(lib.atl_csp_create(self.device, C.byref(cfg), C.byref(h)))
-        self.handle = h
+        self._create(cfg)
 
-    def _fields(self, fields, host):
-        f = _lib.CspFields()
-        keep = []
-        for n in ("influx_direct", "solar_altitude", "solar_azimuth"):
-            a = fields.get(n)
-            if a is None:
-                setattr(f, n, None)
-            elif host:
-                a = self._host(a, f64_ok=n != "influx_direct")
-                keep.append(a)
-                setattr(f, n, a.ctypes.data)
-            else:
-                a = self._dev(a, f64_ok=n != "influx_direct")
-                keep.append(a)
-                setattr(f, n, a.data_ptr())
-        return f, keep
-
-    def reduce(self, plan, fields, t0=0, chunk_steps=0):
-        lib = _lib.load()
-        dev = self._all_device(fields.values())
-        first = fields["influx_direct"]
-        nt = first.shape[0]
-        if nt == 0:
-            return self._empty_like(first, (0, plan.n_bus))
-        f, keep = self._fields(fields, host=not dev)
-        if dev:
-            out = self._out((nt, plan.n_bus), first)
-            _lib.check(lib.atl_csp_reduce(self.handle, plan.handle, C.byref(f), t0, nt, _dptr(out), _stream_ptr()))
-            return out
-        out = np.empty((nt, plan.n_bus), dtype=np.float32)
-        _lib.check(lib.atl_csp_reduce_host(self.handle, plan.handle, C.byref(f), t0, nt, _hptr(out), chunk_steps))
-        return out
-
-    def cells(self, fields, t0=0, timesum=False):
-        lib = _lib.load()
-        first = fields["influx_direct"]
-        nt = first.shape[0]
-        if nt == 0:
-            return self._empty_like(first, (2, self.ny, self.nx) if timesum else (0, self.ny, self.nx))
-        f, keep = self._fields(fields, host=False)
-        torch = _torch()
-        if timesum:
-            out = torch.zeros((2, self.ny, self.nx), dtype=torch.float32, device=first.device)
-            _lib.check(lib.atl_csp_timesum(self.handle, C.byref(f), t0, nt, _dptr(out[0]), _dptr(out[1]), _stream_ptr()))
-        else:
-            out = self._out((nt, self.ny, self.nx), first)
-            _lib.check(lib.atl_csp_cells(self.handle, C.byref(f), t0, nt, _dptr(out), _stream_ptr()))
-        return out
+    _slab = PvOp._slab  # t0 = 0, nt
