@@ -531,6 +531,25 @@ __device__ __forceinline__ void reduce_slots2g_res(const float (&v0)[4], const f
 }  // namespace atl
 
 // Opaque handle definitions shared between translation units.
+
+// Every operator handle (AtlPvOp, AtlWindOp, ...) starts with this: the device it lives on and
+// the grid of its input fields.
+struct AtlOpBase {
+  int device;
+  atl::GridDev grid;
+};
+
+namespace atl {
+// what atl_<op>_op_info reports for every operator
+inline int op_info(const AtlOpBase* op, int32_t* device, int32_t* ny, int32_t* nx) {
+  ATL_REQUIRE(op, "NULL argument");
+  if (device) *device = op->device;
+  if (ny) *ny = op->grid.ny;
+  if (nx) *nx = op->grid.nx;
+  return ATL_OK;
+}
+}  // namespace atl
+
 struct AtlPlan {
   int device;
   atl::GridDev grid;

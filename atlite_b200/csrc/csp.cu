@@ -136,9 +136,7 @@ struct CspPhys {
 
 using namespace atl;
 
-struct AtlCspOp {
-  int device;
-  GridDev grid;
+struct AtlCspOp : AtlOpBase {
   int64_t nt;
   int solar_src, tower, n_alt, n_az;
   float inv_r, dni_thr;
@@ -170,17 +168,29 @@ static CspPhys<VEC> make_phys(const AtlCspOp* op, const AtlCspFields* f, int64_t
   return p;
 }
 
-static bool csp_aligned(const AtlCspFields* f) {
-  return aligned16(f->influx_direct) && aligned16(f->solar_altitude) && aligned16(f->solar_azimuth);
-}
-
-static int csp_check(const AtlCspOp* op, const AtlCspFields* f, int64_t t0, int64_t nt) {
-  ATL_REQUIRE(op && f && f->influx_direct, "NULL argument / influx_direct missing");
-  ATL_REQUIRE(t0 >= 0 && nt >= 0 && t0 + nt <= op->nt, "slab outside the operator's time axis");
-  if (op->solar_src != ATL_SOLAR_COMPUTED)
-    ATL_REQUIRE(f->solar_altitude && f->solar_azimuth, "stored solar position fields missing");
-  return ATL_OK;
-}
+// The CSP operator's part of the shared entry sequence (kernels.cuh: run_entry).
+struct CspBinding {
+  using Op = AtlCspOp;
+  using Fields = AtlCspFields;
+  static int check(const AtlCspOp* op, const AtlCspFields* f, int64_t t0, int64_t nt) {
+    ATL_REQUIRE(op && f && f->influx_direct, "NULL argument / influx_direct missing");
+    ATL_REQUIRE(t0 >= 0 && nt >= 0 && t0 + nt <= op->nt, "slab outside the operator's time axis");
+    if (op->solar_src != ATL_SOLAR_COMPUTED)
+      ATL_REQUIRE(f->solar_altitude && f->solar_azimuth, "stored solar position fields missing");
+    return ATL_OK;
+  }
+  template <class F, class Visit>
+  static void each_field(const AtlCspOp* op, F& f, Visit visit) {
+    const size_t sol = op->solar_src == ATL_SOLAR_STORED_F64 ? 8 : 4;
+    visit(f.influx_direct, 4);
+    visit(f.solar_altitude, sol);
+    visit(f.solar_azimuth, sol);
+  }
+  template <class Run>
+  static int with_phys(const AtlCspOp* op, const AtlCspFields* f, int64_t t0, Run run) {
+    return run([&](auto vec) { return make_phys<decltype(vec)::value>(op, f, t0); });
+  }
+};
 
 extern "C" {
 
@@ -257,45 +267,28 @@ void atl_csp_destroy(AtlCspOp* op) {
 
 int atl_csp_op_info(const AtlCspOp* op, int32_t* device, int32_t* ny, int32_t* nx,
                     int32_t* solar_src) {
-  ATL_REQUIRE(op, "NULL argument");
-  if (device) *device = op->device;
-  if (ny) *ny = op->grid.ny;
-  if (nx) *nx = op->grid.nx;
-  if (solar_src) *solar_src = op->solar_src;
-  return ATL_OK;
+  if (op && solar_src) *solar_src = op->solar_src;
+  return op_info(op, device, ny, nx);
 }
 
 int atl_csp_reduce(const AtlCspOp* op, const AtlPlan* plan, const AtlCspFields* f, int64_t t0,
                    int64_t nt, float* out_dev, void* stream) {
-  int rc = csp_check(op, f, t0, nt);
-  if (rc) return rc;
-  ATL_REQUIRE(plan && out_dev, "NULL argument");
-  ATL_REQUIRE(plan->grid.nx == op->grid.nx && plan->grid.ny == op->grid.ny &&
-                  plan->grid.pitch == op->grid.pitch,
-              "plan / operator grid (or pitch) mismatch");
-  ATL_CUDA(cudaSetDevice(op->device));
-  auto make = [&](auto vec) { return make_phys<decltype(vec)::value>(op, f, t0); };
-  return dispatch_reduce(make, plan, csp_aligned(f), out_dev, nt, (cudaStream_t)stream);
+  return run_entry<CspBinding>(Entry::kReduce, op, plan, f, t0, nt, out_dev, nullptr, stream);
 }
 
 int atl_csp_cells(const AtlCspOp* op, const AtlCspFields* f, int64_t t0, int64_t nt,
                   float* out_dev, void* stream) {
-  int rc = csp_check(op, f, t0, nt);
-  if (rc) return rc;
-  ATL_REQUIRE(out_dev, "NULL argument");
-  ATL_CUDA(cudaSetDevice(op->device));
-  auto make = [&](auto vec) { return make_phys<decltype(vec)::value>(op, f, t0); };
-  return dispatch_cells(make, op->grid, csp_aligned(f), out_dev, nt, false, (cudaStream_t)stream);
+  return run_entry<CspBinding>(Entry::kCells, op, nullptr, f, t0, nt, out_dev, nullptr, stream);
 }
 
 int atl_csp_timesum(const AtlCspOp* op, const AtlCspFields* f, int64_t t0, int64_t nt,
                     float* out_dev, float* count_dev, void* stream) {
-  int rc = csp_check(op, f, t0, nt);
-  if (rc) return rc;
-  ATL_REQUIRE(out_dev, "NULL argument");
-  ATL_CUDA(cudaSetDevice(op->device));
-  auto make = [&](auto vec) { return make_phys<decltype(vec)::value>(op, f, t0); };
-  return dispatch_cells(make, op->grid, csp_aligned(f), out_dev, nt, true, (cudaStream_t)stream, count_dev);
+  return run_entry<CspBinding>(Entry::kTimesum, op, nullptr, f, t0, nt, out_dev, count_dev, stream);
+}
+
+int atl_csp_reduce_host(const AtlCspOp* op, const AtlPlan* plan, const AtlCspFields* f, int64_t t0,
+                        int64_t nt, float* out_host, int64_t chunk_steps) {
+  return run_reduce_host<CspBinding>(op, plan, f, t0, nt, out_host, chunk_steps);
 }
 
 }  // extern "C"

@@ -151,26 +151,35 @@ __global__ void __launch_bounds__(CTA_THREADS, 6)  // latency-bound (ncu: long_s
   }
 }
 
-// Phys adaptor used only by the two-pass fallback (never on the fused path).
 }  // namespace atl
 
 using namespace atl;
 
-struct AtlHeatOp {
-  int device;
-  GridDev grid;
+struct AtlHeatOp : AtlOpBase {
   float thr_k, a, constant;
   int cooling;  // 1: a * (Tmean - threshold)   (convert.py:475-491)
 };
 
-static int upload_days(const int64_t* day_start, int64_t n_days, int32_t** d_out,
-                       cudaStream_t st) {
-  std::vector<int32_t> ds((size_t)n_days + 1);
+// Every argument check of a heat entry point, before any CUDA call.  The day table holds
+// n_days + 1 step offsets, non-decreasing and below 2^31.
+static int check_heat(Entry kind, const AtlHeatOp* op, const AtlPlan* plan, const float* temp,
+                      const int64_t* day_start, int64_t n_days, const float* out) {
+  ATL_REQUIRE(op && temp && day_start && out, "NULL argument");
+  if (kind == Entry::kReduce) {
+    ATL_REQUIRE(plan, "NULL plan");
+    if (int rc = check_plan_grid(op, plan)) return rc;
+  }
+  ATL_REQUIRE(n_days < (1LL << 31), "bad day count");
   for (int64_t i = 0; i <= n_days; ++i) {
     ATL_REQUIRE(day_start[i] >= 0 && day_start[i] < (1LL << 31), "day offset out of range");
     ATL_REQUIRE(i == 0 || day_start[i] >= day_start[i - 1], "day offsets not monotone");
-    ds[(size_t)i] = (int32_t)day_start[i];
   }
+  return ATL_OK;
+}
+
+// The checked day table as int32 in device memory.
+static int upload_days(const int64_t* day_start, int64_t n_days, int32_t** d_out, cudaStream_t st) {
+  const std::vector<int32_t> ds(day_start, day_start + n_days + 1);
   ATL_CUDA(cudaMallocAsync((void**)d_out, ds.size() * 4, st));
   // pageable source: the copy is staged before the call returns
   ATL_CUDA(cudaMemcpyAsync(*d_out, ds.data(), ds.size() * 4, cudaMemcpyHostToDevice, st));
@@ -178,57 +187,9 @@ static int upload_days(const int64_t* day_start, int64_t n_days, int32_t** d_out
   return ATL_OK;
 }
 
-namespace atl {
-// Core launcher: `d_days` is a DEVICE table of n_days+1 step offsets, `base` is
-// subtracted from every entry (so a slab can index into a table uploaded once
-// for the whole time axis; see host_stream.cu).
-int heat_launch_core(int mode, const AtlHeatOp* op, const AtlPlan* plan, const float* temp,
-                     const int32_t* d_days, int32_t base, const int64_t* day_start_host,
-                     int64_t n_days, float* out, cudaStream_t st, float* cnt_out) {
-  ATL_REQUIRE(op && temp && out, "NULL argument");
-  ATL_REQUIRE(n_days >= 0 && n_days < (1LL << 31), "bad day count");
-  if (n_days == 0) return ATL_OK;
-  ATL_CUDA(cudaSetDevice(op->device));
-  PlanDev pd{};
-  int gx;
-  float* det_acc = nullptr;
-  if (mode == 0) {
-    ATL_REQUIRE(plan, "NULL plan");
-    ATL_REQUIRE(plan->grid.nx == op->grid.nx && plan->grid.ny == op->grid.ny &&
-                    plan->grid.pitch == op->grid.pitch,
-                "plan / operator grid (or pitch) mismatch");
-    ATL_CUDA(cudaMemsetAsync(out, 0, (size_t)n_days * plan->n_bus * sizeof(float), st));
-    if (plan->fused) {
-      if (plan->n_active == 0) return ATL_OK;
-      pd = plan->dev();
-      gx = (plan->n_active + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
-      if (deterministic()) {  // see launch_fused: one writer per (slot, day), fixed-order gather
-        ATL_CUDA(cudaMallocAsync((void**)&det_acc, (size_t)n_days * plan->n_slots * sizeof(float), st));
-        ATL_CUDA(cudaMemsetAsync(det_acc, 0, (size_t)n_days * plan->n_slots * sizeof(float), st));
-        pd = plan->dev_partial();
-      }
-    } else {
-      // two-pass fallback: per-cell daily values, then CSR gather
-      ATL_REQUIRE(day_start_host, "two-pass fallback needs the host day table");
-      float* scratch = nullptr;
-      const int64_t S = op->grid.S_out;  // unpadded scratch cube
-      int64_t blk = (256LL << 20) / (S * 4);
-      blk = blk < 1 ? 1 : (blk > n_days ? n_days : blk);
-      ATL_CUDA(cudaMallocAsync((void**)&scratch, (size_t)blk * S * 4, st));
-      int rc = ATL_OK;
-      for (int64_t d = 0; d < n_days && rc == ATL_OK; d += blk) {
-        const int64_t n = n_days - d < blk ? n_days - d : blk;
-        rc = heat_launch_core(1, op, nullptr, temp + (day_start_host[d] - base) * op->grid.S, d_days + d,
-                              (int32_t)day_start_host[d], nullptr, n, scratch, st, nullptr);
-        if (rc == ATL_OK)
-          rc = launch_csr_spmm(plan, scratch, n, out + (size_t)d * plan->n_bus, st);
-      }
-      cudaFreeAsync(scratch, st);
-      return rc;
-    }
-  } else {
-    gx = (op->grid.n_tx * op->grid.n_ty + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
-  }
+// Days [0, n) of the device table `d_days`; `base` is subtracted from its entries, so that a slab of
+// the time axis can index into a table uploaded once for the whole axis (atl_heat_reduce_host).
+static HeatParams heat_params(const AtlHeatOp* op, const float* temp, const int32_t* d_days, int32_t base) {
   HeatParams hp;
   hp.temp = temp;
   hp.day_start = d_days;
@@ -239,6 +200,14 @@ int heat_launch_core(int mode, const AtlHeatOp* op, const AtlPlan* plan, const f
   hp.a = op->a;
   hp.constant = op->constant;
   hp.cooling = op->cooling;
+  return hp;
+}
+
+// k_heat<MODE> over `n_days` days and `n_warps` warp tiles: MODE 0 reduces through `pd` (the
+// plan's active tiles), 1 / 2 store the per-cell daily values / add their sum over all tiles.
+static int launch_heat(int mode, bool vec, const HeatParams& hp, const GridDev& grid, const PlanDev& pd,
+                       int n_warps, int64_t n_days, float* out, float* cnt_out, cudaStream_t st) {
+  const int gx = (n_warps + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
   int db = (int)((n_days * gx + 148LL * 4 * 8 - 1) / (148LL * 4 * 8));
   db = db < 1 ? 1 : (db > 8 ? 8 : db);
   size_t smem = 0;
@@ -246,58 +215,54 @@ int heat_launch_core(int mode, const AtlHeatOp* op, const AtlPlan* plan, const f
     db = HEAT_STAGE;
     smem = StageT<HEAT_STAGE>::kCtaBytes;
   }
-  dim3 grid(gx, (unsigned)((n_days + db - 1) / db));
-  // lane layout: the plan's for the fused reduce, else by grid width / alignment
-  const bool al = aligned16(temp);
-  GridDev gdo = op->grid;
+  GridDev gdo = grid;
   gdo.out_vec = (mode == 1 && gdo.nx % 4 == 0 && aligned16(out)) ? 1 : 0;
-  bool vec = op->grid.pitch % 4 == 0 && al;
-  if (mode == 0) {
-    vec = plan->vec;
-    ATL_REQUIRE(!vec || al,
-                "field pointers must be 16-byte aligned (pitch % 4 == 0 uses 128-bit loads)");
-  }
-  if (vec) {
-    if (mode == 0)
-      k_heat<0, true><<<grid, CTA_THREADS, smem, st>>>(hp, gdo, pd, det_acc ? det_acc : out, nullptr, (int)n_days, db);
-    else if (mode == 1)
-      k_heat<1, true><<<grid, CTA_THREADS, 0, st>>>(hp, gdo, pd, out, nullptr, (int)n_days, db);
-    else
-      k_heat<2, true><<<grid, CTA_THREADS, 0, st>>>(hp, gdo, pd, out, cnt_out, (int)n_days, db);
-  } else {
-    if (mode == 0)
-      k_heat<0, false><<<grid, CTA_THREADS, smem, st>>>(hp, gdo, pd, det_acc ? det_acc : out, nullptr, (int)n_days, db);
-    else if (mode == 1)
-      k_heat<1, false><<<grid, CTA_THREADS, 0, st>>>(hp, gdo, pd, out, nullptr, (int)n_days, db);
-    else
-      k_heat<2, false><<<grid, CTA_THREADS, 0, st>>>(hp, gdo, pd, out, cnt_out, (int)n_days, db);
-  }
+  auto* kern = vec ? (mode == 0 ? k_heat<0, true> : mode == 1 ? k_heat<1, true> : k_heat<2, true>)
+                   : (mode == 0 ? k_heat<0, false> : mode == 1 ? k_heat<1, false> : k_heat<2, false>);
+  kern<<<dim3(gx, (unsigned)((n_days + db - 1) / db)), CTA_THREADS, smem, st>>>(hp, gdo, pd, out, cnt_out,
+                                                                                 (int)n_days, db);
   ++g_launches;
   ATL_CUDA(cudaGetLastError());
-  if (det_acc) {
-    int rc = launch_gather_slots(plan, det_acc, n_days, out, st);
-    cudaFreeAsync(det_acc, st);
-    return rc;
-  }
   return ATL_OK;
 }
 
-int heat_upload_days(const int64_t* day_start, int64_t n_days, int32_t** d_out,
-                     cudaStream_t st) {
-  return upload_days(day_start, n_days, d_out, st);
+// lane layout of the per-cell kernels: by grid width and alignment
+static bool cells_vec(const AtlHeatOp* op, const float* temp) {
+  return op->grid.pitch % 4 == 0 && aligned16(temp);
 }
-}  // namespace atl
 
-static int heat_launch(int mode, const AtlHeatOp* op, const AtlPlan* plan, const float* temp,
-                       const int64_t* day_start, int64_t n_days, float* out, cudaStream_t st,
-                       float* cnt_out = nullptr) {
-  ATL_REQUIRE(op && temp && day_start && out, "NULL argument");
+// (day, bus) sums of days [0, n_days) of the table (see heat_params).
+static int heat_reduce(const AtlHeatOp* op, const AtlPlan* plan, const float* temp, const int32_t* d_days,
+                       int32_t base, int64_t n_days, float* out, cudaStream_t st) {
+  const int n_tiles = op->grid.n_tx * op->grid.n_ty;
+  if (!plan->fused)
+    return two_pass(plan, out, n_days, st, [&](float* scratch, int64_t d0, int64_t n) {
+      return launch_heat(1, cells_vec(op, temp), heat_params(op, temp, d_days + d0, base), op->grid, PlanDev{},
+                         n_tiles, n, scratch, nullptr, st);
+    });
+  ATL_REQUIRE(!plan->vec || aligned16(temp),
+              "field pointers must be 16-byte aligned (pitch % 4 == 0 uses 128-bit loads)");
+  return reduce_into(plan, out, n_days, st, [&](const PlanDev& pd, float* acc) {
+    return launch_heat(0, plan->vec, heat_params(op, temp, d_days, base), op->grid, pd, plan->n_active, n_days,
+                       acc, nullptr, st);
+  });
+}
+
+// atl_heat_reduce / _cells / _timesum
+static int heat_entry(Entry kind, const AtlHeatOp* op, const AtlPlan* plan, const float* temp,
+                      const int64_t* day_start, int64_t n_days, float* out, float* cnt_out, void* stream) {
+  if (int rc = check_heat(kind, op, plan, temp, day_start, n_days, out)) return rc;
   if (n_days <= 0) return ATL_OK;
+  const cudaStream_t st = (cudaStream_t)stream;
   ATL_CUDA(cudaSetDevice(op->device));
   int32_t* d_days = nullptr;
-  int rc = upload_days(day_start, n_days, &d_days, st);
-  if (rc) return rc;
-  rc = heat_launch_core(mode, op, plan, temp, d_days, 0, day_start, n_days, out, st, cnt_out);
+  if (int rc = upload_days(day_start, n_days, &d_days, st)) return rc;
+  int rc;
+  if (kind == Entry::kReduce)
+    rc = heat_reduce(op, plan, temp, d_days, 0, n_days, out, st);
+  else
+    rc = launch_heat(kind == Entry::kCells ? 1 : 2, cells_vec(op, temp), heat_params(op, temp, d_days, 0),
+                     op->grid, PlanDev{}, op->grid.n_tx * op->grid.n_ty, n_days, out, cnt_out, st);
   cudaFreeAsync(d_days, st);
   return rc;
 }
@@ -325,29 +290,43 @@ int atl_heat_create(int device, const AtlHeatConfig* cfg, AtlHeatOp** op_out) {
 void atl_heat_destroy(AtlHeatOp* op) { delete op; }
 
 int atl_heat_op_info(const AtlHeatOp* op, int32_t* device, int32_t* ny, int32_t* nx) {
-  ATL_REQUIRE(op, "NULL argument");
-  if (device) *device = op->device;
-  if (ny) *ny = op->grid.ny;
-  if (nx) *nx = op->grid.nx;
-  return ATL_OK;
+  return op_info(op, device, ny, nx);
 }
 
 int atl_heat_reduce(const AtlHeatOp* op, const AtlPlan* plan, const float* temperature_dev,
                     const int64_t* day_start_host, int64_t n_days, float* out_dev,
                     void* stream) {
-  return heat_launch(0, op, plan, temperature_dev, day_start_host, n_days, out_dev,
-                     (cudaStream_t)stream);
+  return heat_entry(Entry::kReduce, op, plan, temperature_dev, day_start_host, n_days, out_dev, nullptr, stream);
 }
 int atl_heat_cells(const AtlHeatOp* op, const float* temperature_dev,
                    const int64_t* day_start_host, int64_t n_days, float* out_dev, void* stream) {
-  return heat_launch(1, op, nullptr, temperature_dev, day_start_host, n_days, out_dev,
-                     (cudaStream_t)stream);
+  return heat_entry(Entry::kCells, op, nullptr, temperature_dev, day_start_host, n_days, out_dev, nullptr, stream);
 }
 int atl_heat_timesum(const AtlHeatOp* op, const float* temperature_dev,
                      const int64_t* day_start_host, int64_t n_days, float* out_dev,
                      float* count_dev, void* stream) {
-  return heat_launch(2, op, nullptr, temperature_dev, day_start_host, n_days, out_dev,
-                     (cudaStream_t)stream, count_dev);
+  return heat_entry(Entry::kTimesum, op, nullptr, temperature_dev, day_start_host, n_days, out_dev, count_dev,
+                    stream);
+}
+
+// Host temperature: the day table is uploaded once, a slab of days [u0, u0 + n) indexes into it.
+int atl_heat_reduce_host(const AtlHeatOp* op, const AtlPlan* plan, const float* temperature,
+                         const int64_t* day_start, int64_t n_days, float* out_host,
+                         int64_t chunk_days) {
+  ATL_REQUIRE(op && plan && temperature && day_start, "NULL argument");
+  if (int rc = check_host(op, plan, out_host)) return rc;
+  if (int rc = check_heat(Entry::kReduce, op, plan, temperature, day_start, n_days, out_host)) return rc;
+  if (n_days <= 0) return ATL_OK;
+  ATL_CUDA(cudaSetDevice(op->device));
+  int32_t* d_days = nullptr;
+  if (int rc = upload_days(day_start, n_days, &d_days, 0)) return rc;
+  auto launch = [&](const std::vector<void*>& dev, int64_t u0, int64_t n, float* out_dev, cudaStream_t st) {
+    return heat_reduce(op, plan, (const float*)dev[0], d_days + u0, (int32_t)day_start[u0], n, out_dev, st);
+  };
+  const std::vector<SlabField> fields = {{(const char*)temperature, 4}};
+  const int rc = stream_slabs(op, plan, fields, n_days, day_start, chunk_days, out_host, launch);
+  cudaFree(d_days);
+  return rc;
 }
 
 }  // extern "C"

@@ -1,9 +1,11 @@
-// host_stream.cu -- host-buffer entry points: the cutout lives in host memory
-// (NumPy arrays / NetCDF-backed), time slabs are streamed through a
-// double-buffered device ring so H2D copies overlap the fused kernels, and the
-// (time, bus) result is returned in host memory.  This is the call behind the
-// reference-facing `Cutout.pv/wind/heat_demand(...)` when no device-resident
-// copy of the cutout exists (bench.py "e2e").
+// host_stream.cu -- the streaming behind the host-buffer entry points
+// (atl_*_reduce_host): the cutout lives in host memory (NumPy arrays /
+// NetCDF-backed), time slabs are streamed through a double-buffered device ring
+// so H2D copies overlap the fused kernels, and the (time, bus) result is
+// returned in host memory.  This is the call behind the reference-facing
+// `Cutout.pv/wind/heat_demand(...)` when no device-resident copy of the cutout
+// exists (bench.py "e2e").  Nothing here knows an operator: each one lists its
+// fields (kernels.cuh: run_reduce_host, heat.cu).
 //
 // Pinned (cudaHostAlloc / cudaHostRegister'ed) inputs are DMA'd directly;
 // pageable inputs go through a pinned staging ring (memcpy -> async H2D).
@@ -24,15 +26,6 @@
 namespace atl {
 
 constexpr int NBUF = 2;
-
-struct SlabField {
-  const char* host;  // nullptr = unused
-  size_t elem;       // bytes per element
-};
-
-using SlabLaunch =
-    std::function<int(const std::vector<void*>& dev, int64_t t_rel, int64_t n, float* out_dev,
-                      cudaStream_t st)>;
 
 static bool is_pinned(const void* p) {
   cudaPointerAttributes a;
@@ -192,12 +185,13 @@ static void pool_keep_memory(int device) {
 
 // Stream `n_units` time units (steps, or days for heat demand) whose unit u
 // starts at step unit_start(u) through the device ring.
-static int stream_slabs(int device, const std::vector<SlabField>& fields, int64_t S,
-                        int64_t n_units, const int64_t* unit_start /* n_units+1 or NULL */,
-                        int64_t chunk_units, int32_t n_bus, float* out_host,
-                        const SlabLaunch& launch) {
-  ATL_REQUIRE(out_host, "NULL output");
+int stream_slabs(const AtlOpBase* op, const AtlPlan* plan, const std::vector<SlabField>& fields,
+                 int64_t n_units, const int64_t* unit_start, int64_t chunk_units, float* out_host,
+                 const SlabLaunch& launch) {
   if (n_units <= 0) return ATL_OK;
+  const int device = op->device;
+  const int64_t S = op->grid.S;  // == ny * nx: check_host refuses padded operators
+  const int32_t n_bus = plan->n_bus;
   ATL_CUDA(cudaSetDevice(device));
   NumaBind numa(device);
   StagePool& g_stage = stage_pool(device);
@@ -290,7 +284,7 @@ static int stream_slabs(int device, const std::vector<SlabField>& fields, int64_
       SS_CUDA(cudaEventRecord(ev_staged[b], s_copy));
       SS_CUDA(cudaEventRecord(ev_copied[b], s_copy));
       SS_CUDA(cudaStreamWaitEvent(s_comp, ev_copied[b], 0));
-      rc = launch(dev[b], step0, e - u, out_dev + (size_t)u * n_bus, s_comp);
+      rc = launch(dev[b], u, e - u, out_dev + (size_t)u * n_bus, s_comp);
       if (rc != ATL_OK) goto cleanup;
       SS_CUDA(cudaEventRecord(ev_done[b], s_comp));
     }
@@ -326,13 +320,6 @@ cleanup:
 
 using namespace atl;
 
-namespace atl {
-int heat_launch_core(int mode, const AtlHeatOp* op, const AtlPlan* plan, const float* temp,
-                     const int32_t* d_days, int32_t base, const int64_t* day_start_host,
-                     int64_t n_days, float* out, cudaStream_t st, float* cnt_out);
-int heat_upload_days(const int64_t* day_start, int64_t n_days, int32_t** d_out, cudaStream_t st);
-}
-
 extern "C" {
 
 void atl_release_host_staging(void) {
@@ -352,127 +339,6 @@ int atl_device_local_cpus(int device, int32_t* cpus_out, int32_t capacity, int32
     }
   *n_out = n;
   return ATL_OK;
-}
-
-int atl_pv_reduce_host(const AtlPvOp* op, const AtlPlan* plan, const AtlPvFields* f,
-                       int64_t t0, int64_t nt, float* out_host, int64_t chunk_steps) {
-  ATL_REQUIRE(op && plan && f, "NULL argument");
-  int32_t device, ny, nx, solar_src;
-  atl_pv_op_info(op, &device, &ny, &nx, &solar_src);
-  const size_t sol_elem = solar_src == ATL_SOLAR_STORED_F64 ? 8 : 4;
-  std::vector<SlabField> fields = {
-      {(const char*)f->influx_toa, 4},     {(const char*)f->influx_direct, 4},
-      {(const char*)f->influx_diffuse, 4}, {(const char*)f->influx, 4},
-      {(const char*)f->albedo, 4},         {(const char*)f->outflux, 4},
-      {(const char*)f->temperature, 4},    {(const char*)f->humidity, 4},
-      {(const char*)f->solar_altitude, sol_elem},
-      {(const char*)f->solar_azimuth, sol_elem}};
-  auto launch = [&](const std::vector<void*>& d, int64_t t_rel, int64_t n, float* out_dev,
-                    cudaStream_t st) {
-    AtlPvFields df;
-    df.influx_toa = (const float*)d[0];
-    df.influx_direct = (const float*)d[1];
-    df.influx_diffuse = (const float*)d[2];
-    df.influx = (const float*)d[3];
-    df.albedo = (const float*)d[4];
-    df.outflux = (const float*)d[5];
-    df.temperature = (const float*)d[6];
-    df.humidity = (const float*)d[7];
-    df.solar_altitude = d[8];
-    df.solar_azimuth = d[9];
-    return atl_pv_reduce(op, plan, &df, t0 + t_rel, n, out_dev, (void*)st);
-  };
-  AtlPlanInfo pi;
-  atl_plan_info(plan, &pi);
-  return stream_slabs(device, fields, (int64_t)ny * nx, nt, nullptr, chunk_steps, pi.n_bus,
-                      out_host, launch);
-}
-
-int atl_wind_reduce_host(const AtlWindOp* op, const AtlPlan* plan, const AtlWindFields* f,
-                         int64_t nt, float* out_host, int64_t chunk_steps) {
-  ATL_REQUIRE(op && plan && f, "NULL argument");
-  int32_t device, ny, nx;
-  atl_wind_op_info(op, &device, &ny, &nx);
-  std::vector<SlabField> fields = {{(const char*)f->wnd, 4}, {(const char*)f->aux, 4}};
-  auto launch = [&](const std::vector<void*>& d, int64_t, int64_t n, float* out_dev,
-                    cudaStream_t st) {
-    AtlWindFields df;
-    df.wnd = (const float*)d[0];
-    df.aux = (const float*)d[1];
-    return atl_wind_reduce(op, plan, &df, n, out_dev, (void*)st);
-  };
-  AtlPlanInfo pi;
-  atl_plan_info(plan, &pi);
-  return stream_slabs(device, fields, (int64_t)ny * nx, nt, nullptr, chunk_steps, pi.n_bus,
-                      out_host, launch);
-}
-
-int atl_csp_reduce_host(const AtlCspOp* op, const AtlPlan* plan, const AtlCspFields* f,
-                        int64_t t0, int64_t nt, float* out_host, int64_t chunk_steps) {
-  ATL_REQUIRE(op && plan && f, "NULL argument");
-  int32_t device, ny, nx, solar_src;
-  atl_csp_op_info(op, &device, &ny, &nx, &solar_src);
-  const size_t sol_elem = solar_src == ATL_SOLAR_STORED_F64 ? 8 : 4;
-  std::vector<SlabField> fields = {{(const char*)f->influx_direct, 4},
-                                   {(const char*)f->solar_altitude, sol_elem},
-                                   {(const char*)f->solar_azimuth, sol_elem}};
-  auto launch = [&](const std::vector<void*>& d, int64_t t_rel, int64_t n, float* out_dev,
-                    cudaStream_t st) {
-    AtlCspFields df;
-    df.influx_direct = (const float*)d[0];
-    df.solar_altitude = d[1];
-    df.solar_azimuth = d[2];
-    return atl_csp_reduce(op, plan, &df, t0 + t_rel, n, out_dev, (void*)st);
-  };
-  AtlPlanInfo pi;
-  atl_plan_info(plan, &pi);
-  return stream_slabs(device, fields, (int64_t)ny * nx, nt, nullptr, chunk_steps, pi.n_bus,
-                      out_host, launch);
-}
-
-int atl_pointwise_reduce_host(const AtlPointwiseOp* op, const AtlPlan* plan,
-                              const float* field_host, int64_t nt, float* out_host,
-                              int64_t chunk_steps) {
-  ATL_REQUIRE(op && plan && field_host, "NULL argument");
-  int32_t device, ny, nx;
-  atl_pointwise_op_info(op, &device, &ny, &nx);
-  std::vector<SlabField> fields = {{(const char*)field_host, 4}};
-  auto launch = [&](const std::vector<void*>& d, int64_t, int64_t n, float* out_dev,
-                    cudaStream_t st) {
-    return atl_pointwise_reduce(op, plan, (const float*)d[0], n, out_dev, (void*)st);
-  };
-  AtlPlanInfo pi;
-  atl_plan_info(plan, &pi);
-  return stream_slabs(device, fields, (int64_t)ny * nx, nt, nullptr, chunk_steps, pi.n_bus,
-                      out_host, launch);
-}
-
-int atl_heat_reduce_host(const AtlHeatOp* op, const AtlPlan* plan, const float* temperature,
-                         const int64_t* day_start, int64_t n_days, float* out_host,
-                         int64_t chunk_days) {
-  ATL_REQUIRE(op && plan && temperature && day_start, "NULL argument");
-  int32_t device, ny, nx;
-  atl_heat_op_info(op, &device, &ny, &nx);
-  std::vector<SlabField> fields = {{(const char*)temperature, 4}};
-  // one upload of the whole day table; slabs index into it
-  ATL_CUDA(cudaSetDevice(device));
-  int32_t* d_days = nullptr;
-  int rc0 = heat_upload_days(day_start, n_days, &d_days, 0);
-  if (rc0) return rc0;
-  int64_t cursor = 0;  // first day of the slab being launched (slabs are issued in order)
-  auto launch = [&](const std::vector<void*>& d, int64_t, int64_t n, float* out_dev,
-                    cudaStream_t st) {
-    int rc = heat_launch_core(0, op, plan, (const float*)d[0], d_days + cursor,
-                              (int32_t)day_start[cursor], day_start + cursor, n, out_dev, st, nullptr);
-    cursor += n;
-    return rc;
-  };
-  AtlPlanInfo pi;
-  atl_plan_info(plan, &pi);
-  int rc = stream_slabs(device, fields, (int64_t)ny * nx, n_days, day_start, chunk_days,
-                        pi.n_bus, out_host, launch);
-  cudaFree(d_days);
-  return rc;
 }
 
 }  // extern "C"

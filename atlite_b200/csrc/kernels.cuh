@@ -30,7 +30,9 @@
 // buffer (PREFETCH=1: the loads of step t+1 are issued before the arithmetic
 // of step t).
 #pragma once
+#include <functional>
 #include <type_traits>
+#include <vector>
 
 #include "common.cuh"
 
@@ -626,65 +628,47 @@ int launch_staged(const Phys& phys, const AtlPlan* plan, const GridDev& gd, cons
   return ATL_OK;
 }
 
-// Fused path of one slab.  `Phys` must use the plan's lane layout.
-template <class Phys>
-int launch_fused(const Phys& phys, const AtlPlan* plan, float* out, int64_t nt, cudaStream_t st) {
-  const bool det = deterministic() && plan->n_slots > 0;
-  float* acc = out;  // where the per-(slot, step) partial sums are accumulated
-  PlanDev pd = plan->dev();
-  if (det) {
-    ATL_CUDA(cudaMallocAsync((void**)&acc, (size_t)nt * plan->n_slots * sizeof(float), st));
-    pd = plan->dev_partial();
-  }
-  ATL_CUDA(cudaMemsetAsync(acc, 0, (size_t)nt * pd.n_bus * sizeof(float), st));
+// The (unit, bus) target of a fused reduce over `nu` units (time steps, or days).  `kernel(pd, acc)`
+// launches the fused kernel, which accumulates into `acc` through the plan view `pd`: `out`
+// itself, or in deterministic mode a private (unit, slot) buffer with one writer per address
+// that k_gather_slots then sums into `out` in a fixed order.  An empty plan leaves zeros.
+template <class Kernel>
+int reduce_into(const AtlPlan* plan, float* out, int64_t nu, cudaStream_t st, Kernel kernel) {
   if (plan->n_active == 0) {
-    if (det) ATL_CUDA(cudaFreeAsync(acc, st));
-    if (det) ATL_CUDA(cudaMemsetAsync(out, 0, (size_t)nt * plan->n_bus * sizeof(float), st));
+    ATL_CUDA(cudaMemsetAsync(out, 0, (size_t)nu * plan->n_bus * sizeof(float), st));
     return ATL_OK;
   }
-  const int gx = (plan->n_active + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
-  int tb = tuning().tb > 0 ? tuning().tb : pick_tb(gx, nt);
-  const GridDev gd = plan->grid;
-  const int variant = tuning().variant;
-  // ATL_VARIANT: 0 = the functor's own choice (Phys::kStaged), 1 = shuffle reduce against dense
-  // weight vectors, 2 = staged reduce (chunk Phys::kStage), 3 = staged reduce, the other chunk length
-  const bool staged = variant == 0 ? Phys::kStaged : variant != 1;
-  if (!staged) {
-    dim3 grid(gx, (unsigned)((nt + tb - 1) / tb));
-    k_fused_reduce_v1<Phys, Phys::kBatch, Phys::kMinBlocks, 1>
-        <<<grid, CTA_THREADS, Phys::kSmemFloats * sizeof(float), st>>>(phys, gd, pd, acc, (int)nt, tb);
-  } else if (variant == 3) {
-    int rc = launch_staged<Phys, (Phys::kStage == 16 ? 8 : 16)>(phys, plan, gd, pd, acc, nt, tb, gx, st);
-    if (rc) return rc;
-  } else {
-    int rc = launch_staged<Phys, Phys::kStage>(phys, plan, gd, pd, acc, nt, tb, gx, st);
-    if (rc) return rc;
-  }
-  ++g_launches;
-  ATL_CUDA(cudaGetLastError());
+  const bool det = deterministic() && plan->n_slots > 0;
+  float* acc = out;
+  PlanDev pd = plan->dev();
   if (det) {
-    int rc = launch_gather_slots(plan, acc, nt, out, st);
-    cudaFreeAsync(acc, st);
-    return rc;
+    ATL_CUDA(cudaMallocAsync((void**)&acc, (size_t)nu * plan->n_slots * sizeof(float), st));
+    pd = plan->dev_partial();
   }
-  return ATL_OK;
+  cudaError_t e = cudaMemsetAsync(acc, 0, (size_t)nu * pd.n_bus * sizeof(float), st);
+  int rc = e == cudaSuccess ? kernel(pd, acc) : cuda_fail(e, "cudaMemsetAsync(acc)");
+  if (det) {
+    if (rc == ATL_OK) rc = launch_gather_slots(plan, acc, nu, out, st);
+    cudaFreeAsync(acc, st);
+  }
+  return rc;
 }
 
-// Two-pass fallback for matrices that do not tile (e.g. one bus per cell):
-// materialise a block of per-cell values, then CSR-gather it.
-template <class Phys>
-int launch_two_pass(const Phys& phys, const AtlPlan* plan, float* out, int64_t nt,
-                    cudaStream_t st) {
-  const int64_t S = plan->grid.S_out;  // the scratch cube is unpadded
-  int64_t blk = (256LL << 20) / (S * 4);  // <= 256 MiB scratch
+// Two-pass fallback for matrices that do not tile (e.g. one bus per cell): `cells(scratch, u0, n)`
+// writes the per-cell rows of units [u0, u0 + n) into an unpadded scratch block of at most
+// 256 MiB, which a CSR gather then reduces into rows [u0, u0 + n) of `out`.
+template <class Cells>
+int two_pass(const AtlPlan* plan, float* out, int64_t nu, cudaStream_t st, Cells cells) {
+  const int64_t S = plan->grid.S_out;
+  int64_t blk = (256LL << 20) / (S * 4);
   if (blk < 1) blk = 1;
-  if (blk > nt) blk = nt;
+  if (blk > nu) blk = nu;
   float* scratch = nullptr;
   ATL_CUDA(cudaMallocAsync((void**)&scratch, (size_t)blk * S * sizeof(float), st));
-  for (int64_t t = 0; t < nt; t += blk) {
-    const int64_t n = (nt - t < blk) ? nt - t : blk;
-    int rc = launch_cells(phys, plan->grid, scratch, t, t + n, false, st);
-    if (rc == ATL_OK) rc = launch_csr_spmm(plan, scratch, n, out + (size_t)t * plan->n_bus, st);
+  for (int64_t u = 0; u < nu; u += blk) {
+    const int64_t n = (nu - u < blk) ? nu - u : blk;
+    int rc = cells(scratch, u, n);
+    if (rc == ATL_OK) rc = launch_csr_spmm(plan, scratch, n, out + (size_t)u * plan->n_bus, st);
     if (rc != ATL_OK) {
       cudaFreeAsync(scratch, st);
       return rc;
@@ -692,6 +676,43 @@ int launch_two_pass(const Phys& phys, const AtlPlan* plan, float* out, int64_t n
   }
   ATL_CUDA(cudaFreeAsync(scratch, st));
   return ATL_OK;
+}
+
+// Fused path of one slab.  `Phys` must use the plan's lane layout.
+template <class Phys>
+int launch_fused(const Phys& phys, const AtlPlan* plan, float* out, int64_t nt, cudaStream_t st) {
+  return reduce_into(plan, out, nt, st, [&](const PlanDev& pd, float* acc) {
+    const int gx = (plan->n_active + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
+    int tb = tuning().tb > 0 ? tuning().tb : pick_tb(gx, nt);
+    const GridDev gd = plan->grid;
+    const int variant = tuning().variant;
+    // ATL_VARIANT: 0 = the functor's own choice (Phys::kStaged), 1 = shuffle reduce against dense
+    // weight vectors, 2 = staged reduce (chunk Phys::kStage), 3 = staged reduce, the other chunk length
+    const bool staged = variant == 0 ? Phys::kStaged : variant != 1;
+    if (!staged) {
+      dim3 grid(gx, (unsigned)((nt + tb - 1) / tb));
+      k_fused_reduce_v1<Phys, Phys::kBatch, Phys::kMinBlocks, 1>
+          <<<grid, CTA_THREADS, Phys::kSmemFloats * sizeof(float), st>>>(phys, gd, pd, acc, (int)nt, tb);
+    } else if (variant == 3) {
+      int rc = launch_staged<Phys, (Phys::kStage == 16 ? 8 : 16)>(phys, plan, gd, pd, acc, nt, tb, gx, st);
+      if (rc) return rc;
+    } else {
+      int rc = launch_staged<Phys, Phys::kStage>(phys, plan, gd, pd, acc, nt, tb, gx, st);
+      if (rc) return rc;
+    }
+    ++g_launches;
+    ATL_CUDA(cudaGetLastError());
+    return ATL_OK;
+  });
+}
+
+// Two-pass path of one slab: per-cell blocks of the physics, then the CSR gather.
+template <class Phys>
+int launch_two_pass(const Phys& phys, const AtlPlan* plan, float* out, int64_t nt,
+                    cudaStream_t st) {
+  return two_pass(plan, out, nt, st, [&](float* scratch, int64_t t, int64_t n) {
+    return launch_cells(phys, plan->grid, scratch, t, t + n, false, st);
+  });
 }
 
 // Dispatch on the lane layout.  `make(vec_tag)` builds the functor for a layout:
@@ -720,6 +741,94 @@ int dispatch_cells(Make make, const GridDev& gd, bool ptrs_aligned, float* out, 
   if (gd.pitch % 4 == 0 && ptrs_aligned)
     return launch_cells(make(std::true_type{}), gd, out, 0, nt, timesum, st, cnt_out);
   return launch_cells(make(std::false_type{}), gd, out, 0, nt, timesum, st, cnt_out);
+}
+
+// ---------------------------------------------------------------- entry points
+// atl_<op>_reduce / _cells / _timesum of an operator.
+enum class Entry { kReduce, kCells, kTimesum };
+
+inline int check_plan_grid(const AtlOpBase* op, const AtlPlan* plan) {
+  ATL_REQUIRE(plan->grid.nx == op->grid.nx && plan->grid.ny == op->grid.ny &&
+                  plan->grid.pitch == op->grid.pitch,
+              "plan / operator grid (or pitch) mismatch");
+  return ATL_OK;
+}
+
+// Every entry point of a physics-functor operator runs this one sequence: all argument checks,
+// then cudaSetDevice, then the dispatch by kind, so a malformed call is refused before the
+// library touches the device.  The operator's binding `B` supplies
+//   using Op, Fields;                        the handle (derived from AtlOpBase), the field pointers
+//   static int check(const Op*, const Fields*, int64_t t0, int64_t nt);   the operator's own checks
+//   static void each_field(const Op*, F& fields, Visit visit);
+//                                            visit(pointer member, bytes per element) for every field
+//                                            pointer, in one fixed order: the VEC layout needs them all
+//                                            16-byte aligned, host streaming copies and rebinds them
+//   static int with_phys(const Op*, const Fields*, int64_t t0, Run run);
+//                                            run(make) with the functor maker of the operator's
+//                                            compile-time mode, make(vec_tag) -> Phys (dispatch_reduce)
+// Operators without a time axis ignore t0.
+template <class B>
+int run_entry(Entry kind, const typename B::Op* op, const AtlPlan* plan, const typename B::Fields* f,
+              int64_t t0, int64_t nt, float* out, float* cnt_out, void* stream) {
+  if (int rc = B::check(op, f, t0, nt)) return rc;
+  ATL_REQUIRE(out && (plan || kind != Entry::kReduce), "NULL argument");
+  if (kind == Entry::kReduce)
+    if (int rc = check_plan_grid(op, plan)) return rc;
+  ATL_CUDA(cudaSetDevice(op->device));
+  bool al = true;
+  B::each_field(op, *f, [&](const void* p, size_t) { al = al && aligned16(p); });
+  const cudaStream_t st = (cudaStream_t)stream;
+  return B::with_phys(op, f, t0, [&](auto make) {
+    if (kind == Entry::kReduce) return dispatch_reduce(make, plan, al, out, nt, st);
+    return dispatch_cells(make, op->grid, al, out, nt, kind == Entry::kTimesum, st, cnt_out);
+  });
+}
+
+// ---------------------------------------------------------------- host streaming (host_stream.cu)
+// atl_<op>_reduce_host: the fields live in host memory and are streamed in time slabs through a
+// device ring.  The ring holds ny * nx elements per step, so the operator must be unpadded.
+struct SlabField {
+  const char* host;  // nullptr = unused
+  size_t elem;       // bytes per element
+};
+// Reduces units [u0, u0 + n) of the call (steps, or days) whose fields the ring holds at `dev`
+// (one pointer per SlabField, nullptr for unused ones) into `out_dev`.
+using SlabLaunch = std::function<int(const std::vector<void*>& dev, int64_t u0, int64_t n, float* out_dev,
+                                     cudaStream_t st)>;
+
+// The checks every host entry point makes before any CUDA call.
+inline int check_host(const AtlOpBase* op, const AtlPlan* plan, const float* out_host) {
+  ATL_REQUIRE(out_host, "NULL output");
+  if (int rc = check_plan_grid(op, plan)) return rc;
+  ATL_REQUIRE(op->grid.pitch == op->grid.nx,
+              "host entry points take unpadded fields (operator pitch must be nx)");
+  return ATL_OK;
+}
+
+// Streams `n_units` units, unit u starting at step unit_start[u] (n_units + 1 entries; NULL:
+// one step per unit), `chunk_units` per slab (<= 0: about 192 MiB of input), and copies the
+// (unit, bus) result to `out_host`.  The caller has run check_host.
+int stream_slabs(const AtlOpBase* op, const AtlPlan* plan, const std::vector<SlabField>& fields,
+                 int64_t n_units, const int64_t* unit_start, int64_t chunk_units, float* out_host,
+                 const SlabLaunch& launch);
+
+template <class B>
+int run_reduce_host(const typename B::Op* op, const AtlPlan* plan, const typename B::Fields* f, int64_t t0,
+                    int64_t nt, float* out_host, int64_t chunk_steps) {
+  ATL_REQUIRE(op && plan && f, "NULL argument");
+  if (int rc = check_host(op, plan, out_host)) return rc;
+  if (int rc = B::check(op, f, t0, nt)) return rc;
+  std::vector<SlabField> fields;
+  B::each_field(op, *f, [&](const auto& p, size_t elem) { fields.push_back({(const char*)p, elem}); });
+  auto launch = [&](const std::vector<void*>& dev, int64_t u0, int64_t n, float* out_dev, cudaStream_t st) {
+    typename B::Fields df = *f;
+    size_t i = 0;
+    B::each_field(op, df, [&](auto& p, size_t) {
+      p = static_cast<std::remove_reference_t<decltype(p)>>(dev[i++]);  // nullptr stays nullptr
+    });
+    return run_entry<B>(Entry::kReduce, op, plan, &df, t0 + u0, n, out_dev, nullptr, st);
+  };
+  return stream_slabs(op, plan, fields, nt, nullptr, chunk_steps, out_host, launch);
 }
 
 }  // namespace atl

@@ -59,9 +59,7 @@ struct PointwisePhys {
 
 using namespace atl;
 
-struct AtlPointwiseOp {
-  int device;
-  GridDev grid;
+struct AtlPointwiseOp : AtlOpBase {
   float shift, sink, c0, c1, c2;
   int nan_to_zero, poly;
   float* d_scale = nullptr;
@@ -83,6 +81,28 @@ static PointwisePhys<VEC> make_phys(const AtlPointwiseOp* op, const float* field
   p.poly = op->poly;
   return p;
 }
+
+// The pointwise operator's part of the shared entry sequence (kernels.cuh: run_entry): its one
+// field, which the C ABI passes as a bare pointer.  No time axis: t0 is ignored.
+struct PointwiseFields {
+  const float* field;
+};
+struct PointwiseBinding {
+  using Op = AtlPointwiseOp;
+  using Fields = PointwiseFields;
+  static int check(const AtlPointwiseOp* op, const PointwiseFields* f, int64_t, int64_t) {
+    ATL_REQUIRE(op && f->field, "NULL argument");
+    return ATL_OK;
+  }
+  template <class F, class Visit>
+  static void each_field(const AtlPointwiseOp*, F& f, Visit visit) {
+    visit(f.field, 4);
+  }
+  template <class Run>
+  static int with_phys(const AtlPointwiseOp* op, const PointwiseFields* f, int64_t, Run run) {
+    return run([&](auto vec) { return make_phys<decltype(vec)::value>(op, f->field); });
+  }
+};
 
 extern "C" {
 
@@ -125,40 +145,32 @@ void atl_pointwise_destroy(AtlPointwiseOp* op) {
 }
 
 int atl_pointwise_op_info(const AtlPointwiseOp* op, int32_t* device, int32_t* ny, int32_t* nx) {
-  ATL_REQUIRE(op, "NULL argument");
-  if (device) *device = op->device;
-  if (ny) *ny = op->grid.ny;
-  if (nx) *nx = op->grid.nx;
-  return ATL_OK;
+  return op_info(op, device, ny, nx);
 }
 
 int atl_pointwise_reduce(const AtlPointwiseOp* op, const AtlPlan* plan, const float* field_dev,
                          int64_t nt, float* out_dev, void* stream) {
-  ATL_REQUIRE(op && plan && field_dev && out_dev, "NULL argument");
-  ATL_REQUIRE(plan->grid.nx == op->grid.nx && plan->grid.ny == op->grid.ny &&
-                  plan->grid.pitch == op->grid.pitch,
-              "plan / operator grid (or pitch) mismatch");
-  ATL_CUDA(cudaSetDevice(op->device));
-  auto make = [&](auto vec) { return make_phys<decltype(vec)::value>(op, field_dev); };
-  return dispatch_reduce(make, plan, aligned16(field_dev), out_dev, nt, (cudaStream_t)stream);
+  const PointwiseFields f{field_dev};
+  return run_entry<PointwiseBinding>(Entry::kReduce, op, plan, &f, 0, nt, out_dev, nullptr, stream);
 }
 
 int atl_pointwise_cells(const AtlPointwiseOp* op, const float* field_dev, int64_t nt,
                         float* out_dev, void* stream) {
-  ATL_REQUIRE(op && field_dev && out_dev, "NULL argument");
-  ATL_CUDA(cudaSetDevice(op->device));
-  auto make = [&](auto vec) { return make_phys<decltype(vec)::value>(op, field_dev); };
-  return dispatch_cells(make, op->grid, aligned16(field_dev), out_dev, nt, false,
-                        (cudaStream_t)stream);
+  const PointwiseFields f{field_dev};
+  return run_entry<PointwiseBinding>(Entry::kCells, op, nullptr, &f, 0, nt, out_dev, nullptr, stream);
 }
 
 int atl_pointwise_timesum(const AtlPointwiseOp* op, const float* field_dev, int64_t nt,
                           float* out_dev, float* count_dev, void* stream) {
-  ATL_REQUIRE(op && field_dev && out_dev, "NULL argument");
-  ATL_CUDA(cudaSetDevice(op->device));
-  auto make = [&](auto vec) { return make_phys<decltype(vec)::value>(op, field_dev); };
-  return dispatch_cells(make, op->grid, aligned16(field_dev), out_dev, nt, true,
-                        (cudaStream_t)stream, count_dev);
+  const PointwiseFields f{field_dev};
+  return run_entry<PointwiseBinding>(Entry::kTimesum, op, nullptr, &f, 0, nt, out_dev, count_dev, stream);
+}
+
+int atl_pointwise_reduce_host(const AtlPointwiseOp* op, const AtlPlan* plan,
+                              const float* field_host, int64_t nt, float* out_host,
+                              int64_t chunk_steps) {
+  const PointwiseFields f{field_host};
+  return run_reduce_host<PointwiseBinding>(op, plan, &f, 0, nt, out_host, chunk_steps);
 }
 
 }  // extern "C"

@@ -476,9 +476,7 @@ struct PvPhys {
 
 using namespace atl;
 
-struct AtlPvOp {
-  int device;
-  GridDev grid;
+struct AtlPvOp : AtlOpBase {
   int64_t nt;
   int tracking, trigon, clearsky, irr_branch, albedo_src, solar_src, panel_model, output;
   float th_c0, th_c1, th_tstore;
@@ -529,34 +527,53 @@ static PvPhys<MODE, VEC> make_phys(const AtlPvOp* op, const AtlPvFields* f, int6
   return p;
 }
 
-static bool fields_aligned(const AtlPvFields* f) {
-  const void* ps[] = {f->influx_toa, f->influx_direct, f->influx_diffuse, f->influx, f->albedo,
-                      f->outflux,    f->temperature,   f->humidity,       f->solar_altitude,
-                      f->solar_azimuth};
-  for (const void* q : ps)
-    if (!aligned16(q)) return false;
-  return true;
-}
-
-static int check(const AtlPvOp* op, const AtlPvFields* f, int64_t t0, int64_t nt) {
-  ATL_REQUIRE(op && f, "NULL argument");
-  ATL_REQUIRE(t0 >= 0 && nt >= 0 && t0 + nt <= op->nt, "slab outside the operator's time axis");
-  ATL_REQUIRE(f->influx_toa && f->temperature, "influx_toa / temperature field missing");
-  if (op->irr_branch == ATL_IRR_DIRECT_DIFFUSE)
-    ATL_REQUIRE(f->influx_direct && f->influx_diffuse,
-                "Need either influx or influx_direct and influx_diffuse in the dataset.");
-  else {
-    ATL_REQUIRE(f->influx, "influx field missing");
-    if (op->clearsky == ATL_CLEARSKY_ENHANCED) ATL_REQUIRE(f->humidity, "humidity field missing");
+// The PV operator's part of the shared entry sequence (kernels.cuh: run_entry).
+struct PvBinding {
+  using Op = AtlPvOp;
+  using Fields = AtlPvFields;
+  static int check(const AtlPvOp* op, const AtlPvFields* f, int64_t t0, int64_t nt) {
+    ATL_REQUIRE(op && f, "NULL argument");
+    ATL_REQUIRE(t0 >= 0 && nt >= 0 && t0 + nt <= op->nt, "slab outside the operator's time axis");
+    ATL_REQUIRE(f->influx_toa && f->temperature, "influx_toa / temperature field missing");
+    if (op->irr_branch == ATL_IRR_DIRECT_DIFFUSE)
+      ATL_REQUIRE(f->influx_direct && f->influx_diffuse,
+                  "Need either influx or influx_direct and influx_diffuse in the dataset.");
+    else {
+      ATL_REQUIRE(f->influx, "influx field missing");
+      if (op->clearsky == ATL_CLEARSKY_ENHANCED) ATL_REQUIRE(f->humidity, "humidity field missing");
+    }
+    if (op->albedo_src == ATL_ALBEDO_VAR)
+      ATL_REQUIRE(f->albedo, "Need either albedo or outflux as a variable in the dataset.");
+    else
+      ATL_REQUIRE(f->outflux, "outflux field missing");
+    if (op->solar_src != ATL_SOLAR_COMPUTED)
+      ATL_REQUIRE(f->solar_altitude && f->solar_azimuth, "stored solar position fields missing");
+    return ATL_OK;
   }
-  if (op->albedo_src == ATL_ALBEDO_VAR)
-    ATL_REQUIRE(f->albedo, "Need either albedo or outflux as a variable in the dataset.");
-  else
-    ATL_REQUIRE(f->outflux, "outflux field missing");
-  if (op->solar_src != ATL_SOLAR_COMPUTED)
-    ATL_REQUIRE(f->solar_altitude && f->solar_azimuth, "stored solar position fields missing");
-  return ATL_OK;
-}
+  template <class Run>
+  static int with_phys(const AtlPvOp* op, const AtlPvFields* f, int64_t t0, Run run) {
+#define ATL_PV_MODE(M) \
+  case M:              \
+    return run([&](auto vec) { return make_phys<M, decltype(vec)::value>(op, f, t0); });
+    switch (op->mode) { ATL_PV_MODE(0) ATL_PV_MODE(1) ATL_PV_MODE(2) ATL_PV_MODE(3) ATL_PV_MODE(4) }
+#undef ATL_PV_MODE
+    return ATL_ERR_INVALID;
+  }
+  template <class F, class Visit>
+  static void each_field(const AtlPvOp* op, F& f, Visit visit) {
+    const size_t sol = op->solar_src == ATL_SOLAR_STORED_F64 ? 8 : 4;
+    visit(f.influx_toa, 4);
+    visit(f.influx_direct, 4);
+    visit(f.influx_diffuse, 4);
+    visit(f.influx, 4);
+    visit(f.albedo, 4);
+    visit(f.outflux, 4);
+    visit(f.temperature, 4);
+    visit(f.humidity, 4);
+    visit(f.solar_altitude, sol);
+    visit(f.solar_azimuth, sol);
+  }
+};
 
 extern "C" {
 
@@ -698,66 +715,28 @@ void atl_pv_destroy(AtlPvOp* op) {
 
 int atl_pv_op_info(const AtlPvOp* op, int32_t* device, int32_t* ny, int32_t* nx,
                    int32_t* solar_src) {
-  ATL_REQUIRE(op, "NULL argument");
-  if (device) *device = op->device;
-  if (ny) *ny = op->grid.ny;
-  if (nx) *nx = op->grid.nx;
-  if (solar_src) *solar_src = op->solar_src;
-  return ATL_OK;
+  if (op && solar_src) *solar_src = op->solar_src;
+  return op_info(op, device, ny, nx);
 }
 
 int atl_pv_reduce(const AtlPvOp* op, const AtlPlan* plan, const AtlPvFields* f, int64_t t0,
                   int64_t nt, float* out_dev, void* stream) {
-  int rc = check(op, f, t0, nt);
-  if (rc) return rc;
-  ATL_REQUIRE(plan && out_dev, "NULL argument");
-  ATL_REQUIRE(plan->grid.nx == op->grid.nx && plan->grid.ny == op->grid.ny &&
-                  plan->grid.pitch == op->grid.pitch,
-              "plan / operator grid (or pitch) mismatch");
-  ATL_CUDA(cudaSetDevice(op->device));
-  const bool al = fields_aligned(f);
-#define ATL_PV_MODE(M)                                                                  \
-  case M: {                                                                             \
-    auto make = [&](auto vec) { return make_phys<M, decltype(vec)::value>(op, f, t0); }; \
-    return dispatch_reduce(make, plan, al, out_dev, nt, (cudaStream_t)stream);                                                                          \
-  }
-  switch (op->mode) { ATL_PV_MODE(0) ATL_PV_MODE(1) ATL_PV_MODE(2) ATL_PV_MODE(3) ATL_PV_MODE(4) }
-#undef ATL_PV_MODE
-  return ATL_ERR_INVALID;
+  return run_entry<PvBinding>(Entry::kReduce, op, plan, f, t0, nt, out_dev, nullptr, stream);
 }
 
 int atl_pv_cells(const AtlPvOp* op, const AtlPvFields* f, int64_t t0, int64_t nt,
                  float* out_dev, void* stream) {
-  int rc = check(op, f, t0, nt);
-  if (rc) return rc;
-  ATL_REQUIRE(out_dev, "NULL argument");
-  ATL_CUDA(cudaSetDevice(op->device));
-  const bool al = fields_aligned(f);
-#define ATL_PV_MODE(M)                                                                  \
-  case M: {                                                                             \
-    auto make = [&](auto vec) { return make_phys<M, decltype(vec)::value>(op, f, t0); }; \
-    return dispatch_cells(make, op->grid, al, out_dev, nt, false, (cudaStream_t)stream);                                                                          \
-  }
-  switch (op->mode) { ATL_PV_MODE(0) ATL_PV_MODE(1) ATL_PV_MODE(2) ATL_PV_MODE(3) ATL_PV_MODE(4) }
-#undef ATL_PV_MODE
-  return ATL_ERR_INVALID;
+  return run_entry<PvBinding>(Entry::kCells, op, nullptr, f, t0, nt, out_dev, nullptr, stream);
 }
 
 int atl_pv_timesum(const AtlPvOp* op, const AtlPvFields* f, int64_t t0, int64_t nt,
                    float* out_dev, float* count_dev, void* stream) {
-  int rc = check(op, f, t0, nt);
-  if (rc) return rc;
-  ATL_REQUIRE(out_dev, "NULL argument");
-  ATL_CUDA(cudaSetDevice(op->device));
-  const bool al = fields_aligned(f);
-#define ATL_PV_MODE(M)                                                                  \
-  case M: {                                                                             \
-    auto make = [&](auto vec) { return make_phys<M, decltype(vec)::value>(op, f, t0); }; \
-    return dispatch_cells(make, op->grid, al, out_dev, nt, true, (cudaStream_t)stream, count_dev);                                                                          \
-  }
-  switch (op->mode) { ATL_PV_MODE(0) ATL_PV_MODE(1) ATL_PV_MODE(2) ATL_PV_MODE(3) ATL_PV_MODE(4) }
-#undef ATL_PV_MODE
-  return ATL_ERR_INVALID;
+  return run_entry<PvBinding>(Entry::kTimesum, op, nullptr, f, t0, nt, out_dev, count_dev, stream);
+}
+
+int atl_pv_reduce_host(const AtlPvOp* op, const AtlPlan* plan, const AtlPvFields* f, int64_t t0,
+                       int64_t nt, float* out_host, int64_t chunk_steps) {
+  return run_reduce_host<PvBinding>(op, plan, f, t0, nt, out_host, chunk_steps);
 }
 
 }  // extern "C"

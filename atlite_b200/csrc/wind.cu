@@ -269,9 +269,7 @@ struct WindPhys {
 
 using namespace atl;
 
-struct AtlWindOp {
-  int device;
-  GridDev grid;
+struct AtlWindOp : AtlOpBase {
   int method;
   int n_knots, NK;
   float lg2_to, lg2_from, lg2_ratio;
@@ -318,17 +316,38 @@ static WindPhys<VEC, METHOD, LMODE> make_phys(const AtlWindOp* op, const AtlWind
 // compile-time table mode of the operator: 0 generic (binary search / general LUT), 1 + nj lattice,
 // 4 saturating lattice
 static int lut_mode(const AtlWindOp* op) { return op->use_lut == 3 ? 4 : op->use_lut == 2 ? 1 + op->nj : 0; }
-#define ATL_WIND_METHOD_CASES(M)                                                          \
-  ATL_WIND_CASE(M, 0) ATL_WIND_CASE(M, 1) ATL_WIND_CASE(M, 2) ATL_WIND_CASE(M, 3) ATL_WIND_CASE(M, 4)
-#define ATL_WIND_ALL_CASES \
-  ATL_WIND_METHOD_CASES(ATL_WIND_NONE) ATL_WIND_METHOD_CASES(ATL_WIND_LOG) ATL_WIND_METHOD_CASES(ATL_WIND_POWER)
 
-static int check_fields(const AtlWindOp* op, const AtlWindFields* f) {
-  ATL_REQUIRE(op && f && f->wnd, "NULL argument");
-  ATL_REQUIRE(op->method == ATL_WIND_NONE || f->aux,
-              "roughness / wnd_shear_exp field missing for the chosen method");
-  return ATL_OK;
-}
+// The wind operator's part of the shared entry sequence (kernels.cuh: run_entry).  Wind has no
+// time axis: t0 is ignored.
+struct WindBinding {
+  using Op = AtlWindOp;
+  using Fields = AtlWindFields;
+  static int check(const AtlWindOp* op, const AtlWindFields* f, int64_t, int64_t) {
+    ATL_REQUIRE(op && f && f->wnd, "NULL argument");
+    ATL_REQUIRE(op->method == ATL_WIND_NONE || f->aux,
+                "roughness / wnd_shear_exp field missing for the chosen method");
+    return ATL_OK;
+  }
+  template <class F, class Visit>
+  static void each_field(const AtlWindOp*, F& f, Visit visit) {
+    visit(f.wnd, 4);
+    visit(f.aux, 4);
+  }
+  template <class Run>
+  static int with_phys(const AtlWindOp* op, const AtlWindFields* f, int64_t, Run run) {
+#define ATL_WIND_CASE(M, L) \
+  case 8 * M + L:           \
+    return run([&](auto vec) { return make_phys<decltype(vec)::value, M, L>(op, f); });
+#define ATL_WIND_METHOD_CASES(M) \
+  ATL_WIND_CASE(M, 0) ATL_WIND_CASE(M, 1) ATL_WIND_CASE(M, 2) ATL_WIND_CASE(M, 3) ATL_WIND_CASE(M, 4)
+    switch (8 * op->method + lut_mode(op)) {
+      ATL_WIND_METHOD_CASES(ATL_WIND_NONE) ATL_WIND_METHOD_CASES(ATL_WIND_LOG) ATL_WIND_METHOD_CASES(ATL_WIND_POWER)
+    }
+#undef ATL_WIND_METHOD_CASES
+#undef ATL_WIND_CASE
+    return ATL_ERR_INVALID;
+  }
+};
 
 // Host-side tables of a power curve (shared by atl_wind_create and the host
 // evaluator atl_wind_curve_eval_host the CPU tests use).
@@ -790,65 +809,27 @@ int atl_wind_curve_info_host(const double* V, const double* POW_norm, int32_t n_
 }
 
 int atl_wind_op_info(const AtlWindOp* op, int32_t* device, int32_t* ny, int32_t* nx) {
-  ATL_REQUIRE(op, "NULL argument");
-  if (device) *device = op->device;
-  if (ny) *ny = op->grid.ny;
-  if (nx) *nx = op->grid.nx;
-  return ATL_OK;
+  return op_info(op, device, ny, nx);
 }
 
 int atl_wind_reduce(const AtlWindOp* op, const AtlPlan* plan, const AtlWindFields* f,
                     int64_t nt, float* out_dev, void* stream) {
-  int rc = check_fields(op, f);
-  if (rc) return rc;
-  ATL_REQUIRE(plan && out_dev, "NULL argument");
-  ATL_REQUIRE(plan->grid.nx == op->grid.nx && plan->grid.ny == op->grid.ny &&
-                  plan->grid.pitch == op->grid.pitch,
-              "plan / operator grid (or pitch) mismatch");
-  ATL_CUDA(cudaSetDevice(op->device));
-  const bool al = aligned16(f->wnd) && aligned16(f->aux);
-#define ATL_WIND_CASE(M, L)                                                               \
-  case 8 * M + L: {                                                                       \
-    auto make = [&](auto vec) { return make_phys<decltype(vec)::value, M, L>(op, f); };   \
-    return dispatch_reduce(make, plan, al, out_dev, nt, (cudaStream_t)stream);            \
-  }
-  switch (8 * op->method + lut_mode(op)) { ATL_WIND_ALL_CASES }
-#undef ATL_WIND_CASE
-  return ATL_ERR_INVALID;
+  return run_entry<WindBinding>(Entry::kReduce, op, plan, f, 0, nt, out_dev, nullptr, stream);
 }
 
 int atl_wind_cells(const AtlWindOp* op, const AtlWindFields* f, int64_t nt, float* out_dev,
                    void* stream) {
-  int rc = check_fields(op, f);
-  if (rc) return rc;
-  ATL_REQUIRE(out_dev, "NULL argument");
-  ATL_CUDA(cudaSetDevice(op->device));
-  const bool al = aligned16(f->wnd) && aligned16(f->aux);
-#define ATL_WIND_CASE(M, L)                                                               \
-  case 8 * M + L: {                                                                       \
-    auto make = [&](auto vec) { return make_phys<decltype(vec)::value, M, L>(op, f); };   \
-    return dispatch_cells(make, op->grid, al, out_dev, nt, false, (cudaStream_t)stream);  \
-  }
-  switch (8 * op->method + lut_mode(op)) { ATL_WIND_ALL_CASES }
-#undef ATL_WIND_CASE
-  return ATL_ERR_INVALID;
+  return run_entry<WindBinding>(Entry::kCells, op, nullptr, f, 0, nt, out_dev, nullptr, stream);
 }
 
 int atl_wind_timesum(const AtlWindOp* op, const AtlWindFields* f, int64_t nt, float* out_dev,
                      float* count_dev, void* stream) {
-  int rc = check_fields(op, f);
-  if (rc) return rc;
-  ATL_REQUIRE(out_dev, "NULL argument");
-  ATL_CUDA(cudaSetDevice(op->device));
-  const bool al = aligned16(f->wnd) && aligned16(f->aux);
-#define ATL_WIND_CASE(M, L)                                                               \
-  case 8 * M + L: {                                                                       \
-    auto make = [&](auto vec) { return make_phys<decltype(vec)::value, M, L>(op, f); };   \
-    return dispatch_cells(make, op->grid, al, out_dev, nt, true, (cudaStream_t)stream, count_dev);  \
-  }
-  switch (8 * op->method + lut_mode(op)) { ATL_WIND_ALL_CASES }
-#undef ATL_WIND_CASE
-  return ATL_ERR_INVALID;
+  return run_entry<WindBinding>(Entry::kTimesum, op, nullptr, f, 0, nt, out_dev, count_dev, stream);
+}
+
+int atl_wind_reduce_host(const AtlWindOp* op, const AtlPlan* plan, const AtlWindFields* f,
+                         int64_t nt, float* out_host, int64_t chunk_steps) {
+  return run_reduce_host<WindBinding>(op, plan, f, 0, nt, out_host, chunk_steps);
 }
 
 }  // extern "C"

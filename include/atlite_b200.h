@@ -33,7 +33,8 @@
  *     row-padded (pitch = round_up(nx, 4), padding contents arbitrary) so that
  *     the 128-bit kernels apply; operator and plan must be created with the same
  *     pitch.  Host entry points (*_reduce_host) always take unpadded arrays
- *     (pitch = nx operators); per-cell OUTPUTS are never padded.
+ *     (pitch = nx operators; a padded one is refused with ATL_ERR_INVALID);
+ *     per-cell OUTPUTS are never padded.
  *   - Pointers named *_dev are device pointers on the operator's device, those
  *     named *_host are host pointers.  Small tables (coordinates, time axis,
  *     power curve) are always host pointers and are copied at create time.
